@@ -4,6 +4,7 @@ bench.py -- megapixels/second through pipe_color2d_slic_features_model_graphcut 
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path (oracle port) on host cores
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's (segm, segm_soft) to DIR/*.npy
 
 Workload (BASELINE.json configs[1], SURVEY.md section 8d "config 2"): one synthetic 2048x2048 RGB float64 image per
 GPU per step -- Voronoi regions with 3 class means + gaussian noise, sp_size 29 (4 987 seeds), colour-mean descriptors,
@@ -187,6 +188,20 @@ class ClockSampler(object):
                 'samples': len(sm)}
 
 
+#: pixels of segm_soft that --dump-outputs writes: the whole [H, W, K] float64 array is 100 MB, the sample 25 MB
+DUMP_SOFT_PIXELS = 1 << 20
+
+
+def dump_outputs(out_dir, segm, soft):
+    """what the headline path returns, for comparing two builds output for output: the label map whole (float32 holds every label
+    exactly) and a fixed, seeded sample of segm_soft's pixels (float64) with their flat pixel indices"""
+    os.makedirs(out_dir, exist_ok=True)
+    idx = np.sort(np.random.RandomState(0).choice(segm.size, DUMP_SOFT_PIXELS, replace=False))
+    np.save(os.path.join(out_dir, 'segm.npy'), segm.astype(np.float32))
+    np.save(os.path.join(out_dir, 'segm_soft_sample.npy'), soft.reshape(segm.size, -1)[idx].astype(np.float64))
+    np.save(os.path.join(out_dir, 'segm_soft_sample_index.npy'), idx.astype(np.float64))
+
+
 def dist_env():
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
@@ -241,8 +256,6 @@ class ReferencePool(object):
 
     def __init__(self, n_images, workers, first_seed=1000):
         import multiprocessing as mp
-        import oracle
-        oracle.build()
         del _REF_IMAGES[:]
         _REF_IMAGES.extend(synth_image(first_seed + i) for i in range(n_images))
         self.n, self.workers = n_images, workers
@@ -375,8 +388,10 @@ def run_ours(args):
         sampler.start()
     # timed region 1 (the `value`): the device part replayed as one CUDA graph per image (pipelines._run_resident_graph)
     n0 = lib.isb_launch_count()
-    ms_res, _ = timed(step_resident, args.steps)
+    ms_res, (d_segm, d_soft) = timed(step_resident, args.steps)
     launches = lib.isb_launch_count() - n0
+    # copied now: the passes below refill the same engine buffers
+    outputs = (d_segm.cpu().numpy(), d_soft.cpu().numpy()) if args.dump_outputs and rank == 0 else None
     # timed region 2 (same steps, eager launches): per-stage CUDA events on the launching stream -> `stages` and the roofline
     pipelines.USE_CUDA_GRAPHS = False
     step_resident()
@@ -400,7 +415,7 @@ def run_ours(args):
         return None
 
     batch_once()
-    ms_batch, _ = timed(batch_once, 2)
+    ms_batch, _ = timed(batch_once, args.steps)
     clocks = sampler.stop() if rank == 0 else None
 
     stages = {lib.isb_profile_stage_name(i).decode(): {'ms_per_step': ms_arr[i] / args.steps, 'launches_per_step': cnt_arr[i] / args.steps}
@@ -434,7 +449,7 @@ def run_ours(args):
                 'd2h_bytes_per_step': int(segm.nbytes + soft.nbytes), 'source': 'pinned host ndarray'},
         'e2e_pageable': {'value': world * args.steps * mpix / (ms_page / 1e3), 'unit': 'MPix/s', 'ms_per_step': ms_page / args.steps,
                          'source': 'ordinary (pageable) numpy array, as a caller of the reference API would pass it'},
-        'e2e_batch': {'value': world * 2 * nbatch * mpix / (ms_batch / 1e3), 'unit': 'MPix/s', 'images_per_call': nbatch,
+        'e2e_batch': {'value': world * args.steps * nbatch * mpix / (ms_batch / 1e3), 'unit': 'MPix/s', 'images_per_call': nbatch,
                       'note': 'segment_images_batch: same host-in/host-out path, copies of consecutive images overlapped on 3 streams'},
         'gpu_launches': int(launches),
         'roofline': {'kernel': 'k_assign (slic_assign)', 'bound': 'hbm', 'achieved': achieved, 'peak': peak, 'unit': 'GB/s',
@@ -467,6 +482,8 @@ def run_ours(args):
         line['parity'] = {'image': 'synth_image(1000), 2048x2048', 'superpixel_label_map_identical': same,
                           'nb_superpixels': int(d_slic.max()) + 1,
                           'features_max_abs_err': float(np.max(np.abs(o_fts - d_fts))) if same and o_fts.shape == d_fts.shape else None}
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, *outputs)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -728,7 +745,13 @@ def main():
     ap.add_argument('--workload', default='config2', choices=['config2', 'config3', 'config4', 'config5'],
                     help='config2 = the headline line (default); config5 = one 8192x8192 image banded over the GPUs (extra)')
     ap.add_argument('--tiled-side', type=int, default=8192)
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step of the headline path returned to DIR/<name>.npy (see dump_outputs)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and (args.impl != 'ours' or args.workload != 'config2'):
+        ap.error('--dump-outputs applies to the headline workload (--impl ours --workload config2)')
     if args.impl == 'reference':
         run_reference(args)
     elif args.workload == 'config5':

@@ -1,10 +1,15 @@
 """GPU parity tests proper: the CUDA path (through the C-ABI) against the CPU oracle on the same seeded inputs."""
+import os
+
 import numpy as np
 import pytest
 
 from conftest import synth_disc, synth_regions
 
 pytestmark = pytest.mark.gpu
+
+#: outputs of the reference's Cython module for inputs built below (tests/golden/make_cython_goldens.py)
+REF_CYTHON = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'reference_cython.npz'))
 
 
 @pytest.fixture(scope='module')
@@ -55,10 +60,7 @@ def test_color_stats_match_oracle_and_reference_module(oracle):
         for name, fn_o in (('mean', oracle.color2d_mean), ('energy', oracle.color2d_energy), ('std', oracle.color2d_std)):
             got = getattr(ds, 'cython_img2d_color_%s' % name)(im, seg)
             np.testing.assert_allclose(got, fn_o(im, seg), rtol=1e-6, atol=1e-9)
-    fc = oracle.ref_features_cython()
-    if fc is not None:
-        ref = np.array(fc.computeColorImage2dEnergy(img.astype(np.float32), seg.astype(np.int32)))
-        np.testing.assert_allclose(ds.cython_img2d_color_energy(img, seg), ref, rtol=1e-6, atol=1e-9)
+    np.testing.assert_allclose(ds.cython_img2d_color_energy(img, seg), REF_CYTHON['slic_energy'], rtol=1e-6, atol=1e-9)
     fts, names = ds.compute_image2d_color_statistic(img, seg, ('mean', 'std', 'energy', 'meanGrad'))
     want = oracle.image2d_color_statistic(img, seg, ('mean', 'std', 'energy', 'meanGrad'))
     assert fts.shape == (seg.max() + 1, 12) and len(names) == 12
@@ -322,7 +324,7 @@ def test_config1_reference_cpu_case(oracle):
 
 def test_remaining_native_functions(oracle):
     """gray 3-D statistics, label histogram and ray features of imsegm/features_cython.pyx (:144-282): doctest goldens of
-    imsegm/descriptors.py:470-478, :1479-1485, :1641-1653, the oracle, and the reference module compiled unchanged.
+    imsegm/descriptors.py:470-478, :1479-1485, :1641-1653, the oracle, and stored outputs of the reference module compiled unchanged.
     Ray distances: 1e-5 relative against the compiled reference (it is built with -ffast-math, its last float ulp is
     compiler dependent); exact against the oracle and against the integer goldens."""
     from pyimsegm_b200 import descriptors as ds
@@ -351,16 +353,13 @@ def test_remaining_native_functions(oracle):
     assert ds.cython_ray_features_seg2d(seg, (60, 40), 30).astype(int).tolist() == [74, 55, 28, 10, 5, 4, 4, 5, 9, 30, 57, 75]
     assert ds.cython_ray_features_seg2d(seg, (40, 60), 20).astype(int).tolist() == \
         [54, 57, 58, 55, 50, 43, 38, 31, 26, 24, 22, 22, 23, 26, 29, 34, 41, 48]
-    fc = oracle.ref_features_cython()
     noise = rng.rand(40, 60) < 0.08
     pos = np.stack([rng.randint(0, 40, 25), rng.randint(0, 60, 25)], 1)
     for edge, e in (('up', 1), ('down', -1)):
         got = ds.cython_ray_features_seg2d(noise, pos, 7.5, edge)
-        for p, g in zip(pos, got):
+        for p, g, ref in zip(pos, got, REF_CYTHON['rays_' + edge]):
             assert np.array_equal(g, oracle.ray_features2d(noise, p, 7.5, e))
-            if fc is not None:
-                ref = np.array(fc.computeRayFeaturesBinary2d(noise.astype(np.int8), np.array(p, dtype=np.int32), 7.5, e))
-                np.testing.assert_allclose(g, ref, rtol=1e-5)
+            np.testing.assert_allclose(g, ref, rtol=1e-5)
 
 
 @pytest.mark.parametrize('sp_size,regul,shape', [(4, 0.3, (96, 128)), (5, 0.15, (77, 101)), (60, 0.2, (200, 260)), (9, 0.5, (33, 47))])
