@@ -11,7 +11,7 @@ import logging
 
 import numpy as np
 
-from .engine import FLAG_BITS, get_engine
+from .engine import FLAG_BITS, dtype_code, flag_bits, get_engine
 from .utilities import ImageDimensionError
 
 #: kept for API compatibility with the reference (descriptors.py:25-33); the native path here is CUDA and it
@@ -145,8 +145,6 @@ def numpy_img2d_color_energy(img, seg):
 
 def _device_median(img, seg, channels):
     """per-label median of every channel on the device (``isb_segment_median``: counting sort by label + radix select)"""
-    import ctypes as C
-    from . import _lib
     eng = get_engine()
     img = _device_dtype(img)
     n_px = int(seg.size)
@@ -154,11 +152,8 @@ def _device_median(img, seg, channels):
     d_img = eng.to_device(img, 'median_img')
     d_seg = eng.to_device(np.ascontiguousarray(seg, dtype=np.int32), 'seg_in')
     out = eng.buf('median_out', (nb, channels), eng.torch.float64)
-    wsb = eng.lib.isb_segment_median_workspace_bytes(C.c_longlong(n_px), nb)
-    ws = eng.buf('ws_median', (wsb,), eng.torch.uint8)
-    code = _lib.DTYPE_CODES[str(img.dtype)]
-    _lib.check(eng.lib.isb_segment_median(_lib.ptr(d_img), code, _lib.ptr(d_seg), C.c_longlong(n_px), channels, nb, _lib.ptr(out), _lib.ptr(ws),
-                                          C.c_size_t(wsb), _lib.stream_ptr()))
+    ws, wsb = eng.workspace('ws_median', 'segment_median_workspace_bytes', n_px, nb)
+    eng.call('segment_median', d_img, dtype_code(img.dtype), d_seg, n_px, channels, nb, out, ws, wsb)
     return eng.to_host(out).copy()
 
 
@@ -171,20 +166,16 @@ def numpy_img2d_color_median(img, seg):
 
 
 def _device_gray_stats(img, seg, flags):
-    import ctypes as C
-    from . import _lib
     img, seg = _device_dtype(img), np.asarray(seg)
     _check_gray_image_segm(img, seg)
     eng = get_engine()
     nb = int(seg.max()) + 1
     d_img = eng.to_device(img, 'image_gray')
     d_seg = eng.to_device(seg.astype(np.int32, copy=False), 'seg_in')
-    bits = sum(FLAG_BITS[f] for f in flags)
-    feat = eng.buf('feat_gray', (nb, len(flags)), eng.torch.float64)
-    wsb = eng.lib.isb_gray_stats_workspace_bytes(nb)
-    ws = eng.buf('ws_gray', (wsb,), eng.torch.uint8)
-    _lib.check(eng.lib.isb_gray_stats(_lib.ptr(d_img), _lib.DTYPE_CODES[str(img.dtype)], _lib.ptr(d_seg), C.c_longlong(img.size), nb, bits,
-                                      _lib.ptr(feat), len(flags), 0, _lib.ptr(ws), C.c_size_t(wsb), _lib.stream_ptr()))
+    bits, n = flag_bits(flags)
+    feat = eng.buf('feat_gray', (nb, n), eng.torch.float64)
+    ws, wsb = eng.workspace('ws_gray', 'gray_stats_workspace_bytes', nb)
+    eng.call('gray_stats', d_img, dtype_code(img.dtype), d_seg, img.size, nb, bits, feat, n, 0, ws, wsb)
     return eng.to_host(feat).copy()
 
 
@@ -205,8 +196,6 @@ def cython_img3d_gray_std(img, seg, mean=None):
 
 def cython_label_hist_seg2d(segm_select, struc_elem, nb_labels):
     """ histogram of the labels under a structuring element (reference descriptors.py:1479-1498) """
-    import ctypes as C
-    from . import _lib
     segm_select, struc_elem = np.array(segm_select, dtype=float), np.asarray(struc_elem)
     if segm_select.shape != struc_elem.shape:
         raise ValueError('segm. %r and mask %r sizes do not match' % (segm_select.shape, struc_elem.shape))
@@ -215,8 +204,7 @@ def cython_label_hist_seg2d(segm_select, struc_elem, nb_labels):
     d_a = eng.to_device(segm_select.astype(np.int16), 'hist_segm')
     d_b = eng.to_device(struc_elem.astype(np.int16), 'hist_selem')
     hist = eng.buf('hist_out', (int(nb_labels),), eng.torch.int32)
-    _lib.check(eng.lib.isb_label_hist_2d(_lib.ptr(d_a), _lib.ptr(d_b), segm_select.shape[0], segm_select.shape[1], int(nb_labels),
-                                         _lib.ptr(hist), _lib.stream_ptr()))
+    eng.call('label_hist_2d', d_a, d_b, segm_select.shape[0], segm_select.shape[1], int(nb_labels), hist)
     return eng.to_host(hist).astype(float)
 
 
@@ -233,8 +221,6 @@ def cython_ray_features_seg2d(seg_binary, position, angle_step=5., edge='up'):
 
     :return ndarray: ray distances, float32 [n_angles] (or [n, n_angles])
     """
-    import ctypes as C
-    from . import _lib
     edge_int = {'down': -1, 'up': 1}[edge]
     seg = np.array(seg_binary, dtype=np.int8)
     pos = np.atleast_2d(np.array(position, dtype=np.int32))
@@ -243,8 +229,7 @@ def cython_ray_features_seg2d(seg_binary, position, angle_step=5., edge='up'):
     d_seg, d_pos = eng.to_device(seg, 'ray_seg'), eng.to_device(pos, 'ray_pos')
     d_s, d_c = eng.to_device(sin_a, 'ray_sin'), eng.to_device(cos_a, 'ray_cos')
     out = eng.buf('ray_out', (len(pos), len(sin_a)), eng.torch.float32)
-    _lib.check(eng.lib.isb_ray_features_2d(_lib.ptr(d_seg), seg.shape[0], seg.shape[1], _lib.ptr(d_pos), len(pos), _lib.ptr(d_s), _lib.ptr(d_c),
-                                           len(sin_a), edge_int, _lib.ptr(out), _lib.stream_ptr()))
+    eng.call('ray_features_2d', d_seg, seg.shape[0], seg.shape[1], d_pos, len(pos), d_s, d_c, len(sin_a), edge_int, out)
     res = eng.to_host(out).copy()
     return res[0] if np.ndim(position) == 1 else res
 
@@ -362,7 +347,6 @@ def compute_img_filter_response2d(img, filter_battery):
 
 def compute_img_filter_response3d(img, filter_battery):
     """ :func:`compute_img_filter_response2d` of every slice ``img[i]`` in one launch (reference descriptors.py:969-983) """
-    from . import _lib
     filter_battery = np.ascontiguousarray(filter_battery, dtype=np.float64)
     if filter_battery.ndim != 3:
         raise ValueError('wrong battery dim %r' % (filter_battery.shape, ))
@@ -373,14 +357,13 @@ def compute_img_filter_response3d(img, filter_battery):
     d_img = eng.to_device(img, 'resp_img')
     d_ker = eng.to_device(filter_battery, 'resp_kernels')
     out = eng.buf('resp_out', img.shape, eng.torch.float64)
-    _lib.check(eng.lib.isb_filter_response_2d(_lib.ptr(d_img), img.shape[0], img.shape[1], img.shape[2], _lib.ptr(d_ker), filter_battery.shape[0],
-                                              filter_battery.shape[1], filter_battery.shape[2], _lib.ptr(out), _lib.stream_ptr()))
+    eng.call('filter_response_2d', d_img, img.shape[0], img.shape[1], img.shape[2], d_ker, filter_battery.shape[0], filter_battery.shape[1],
+             filter_battery.shape[2], out)
     return eng.to_host(out).copy()
 
 
 def _gauss_smooth_slices(stack, sigma):
     """scipy ``gaussian_filter(slice, sigma)`` of every 2-D slice of a float64 stack [n, H, W], FP64 on the device"""
-    from . import _lib
     from .engine import gaussian_half_kernel
     w_half, radius = gaussian_half_kernel(sigma)
     eng = get_engine()
@@ -388,8 +371,7 @@ def _gauss_smooth_slices(stack, sigma):
     d_w = eng.to_device(w_half, 'smooth_w')
     tmp = eng.buf('smooth_tmp', stack.shape, eng.torch.float64)
     out = eng.buf('smooth_out', stack.shape, eng.torch.float64)
-    _lib.check(eng.lib.isb_gaussian_filter_2d(_lib.ptr(d_img), stack.shape[0], stack.shape[1], stack.shape[2], _lib.ptr(d_w), radius,
-                                              _lib.ptr(tmp), _lib.ptr(out), _lib.stream_ptr()))
+    eng.call('gaussian_filter_2d', d_img, stack.shape[0], stack.shape[1], stack.shape[2], d_w, radius, tmp, out)
     return eng.to_host(out).copy()
 
 
@@ -497,8 +479,6 @@ def _device_label_hists(segm, positions, nb_labels, diameters=None, struc_elem=N
     """label histograms under discs (``diameters``) or one explicit structuring element about every position, one launch
     (``isb_disc_label_hist``).  ``segm`` is [H, W] labels or [H, W, K] per-label maps.
     Returns (hist [n_pos, n_elems, nb_labels], sizes [n_pos, n_elems])."""
-    import ctypes as C
-    from . import _lib
     segm = np.asarray(segm)
     pos = np.ascontiguousarray(np.atleast_2d(np.asarray(positions)).astype(np.int32))
     if pos.shape[1] != 2:
@@ -527,8 +507,7 @@ def _device_label_hists(segm, positions, nb_labels, diameters=None, struc_elem=N
         n_el = len(diam)
     hist = eng.buf('hist_out64', (len(pos), n_el, int(nb_labels)), torch.float64)
     sizes = eng.buf('hist_sizes', (len(pos), n_el), torch.float64)
-    _lib.check(eng.lib.isb_disc_label_hist(_lib.ptr(d_seg), _lib.ptr(d_proba), H, W, _lib.ptr(d_pos), len(pos), _lib.ptr(d_diam), n_el,
-                                           _lib.ptr(d_sel), mh, mw, int(nb_labels), _lib.ptr(hist), _lib.ptr(sizes), _lib.stream_ptr()))
+    eng.call('disc_label_hist', d_seg, d_proba, H, W, d_pos, len(pos), d_diam, n_el, d_sel, mh, mw, int(nb_labels), hist, sizes)
     return eng.to_host(hist).copy(), eng.to_host(sizes).copy()
 
 
@@ -681,7 +660,6 @@ def compute_ray_features_positions(segm, list_positions, angle_step=5., border_l
 def binary_opening_disk(mask, radius):
     """ morphological opening of a binary 2-D mask with a disc of ``radius`` pixels, borders reflected -- what the reference gets
     from ``skimage.morphology.opening(mask, morphology.disk(radius))`` (descriptors.py:1873-1876); ``isb_binary_opening_disk`` """
-    from . import _lib
     mask = np.ascontiguousarray(mask, dtype=np.uint8)
     if mask.ndim != 2:
         raise ValueError('expected a 2-D mask, got shape %r' % (mask.shape, ))
@@ -689,8 +667,7 @@ def binary_opening_disk(mask, radius):
     d_in = eng.to_device(mask, 'morph_in')
     tmp = eng.buf('morph_tmp', mask.shape, eng.torch.uint8)
     out = eng.buf('morph_out', mask.shape, eng.torch.uint8)
-    _lib.check(eng.lib.isb_binary_opening_disk(_lib.ptr(d_in), mask.shape[0], mask.shape[1], int(radius), _lib.ptr(tmp), _lib.ptr(out),
-                                               _lib.stream_ptr()))
+    eng.call('binary_opening_disk', d_in, mask.shape[0], mask.shape[1], int(radius), tmp, out)
     return eng.to_host(out).astype(bool)
 
 

@@ -3,8 +3,8 @@ Device-resident driver of the SLIC -> descriptors -> GraphCut hot path.
 
 Everything here is plumbing: torch tensors are used purely as device-memory containers and every computation is
 a call into ``libimsegm_b200.so`` through the C-ABI (``include/imsegm_b200.h``).  No torch op touches the data
-path.  The numpy-facing modules (``superpixels``, ``descriptors``, ``graph_cuts``, ``pipelines``) are thin
-wrappers over this class.
+path.  The numpy-facing modules (``superpixels``, ``descriptors``, ``graph_cuts``, ``pipelines``, ``tiled``, ``texture``) are thin
+wrappers over this class, and :meth:`Engine.call` is the only way they reach the library.
 """
 import ctypes as C
 
@@ -12,10 +12,39 @@ import numpy as np
 
 from . import _lib
 
+_DOUBLE_P = C.POINTER(C.c_double)
 FLAG_BITS = {'mean': 1, 'std': 2, 'energy': 4}
+#: initial capacity of a device edge table, in edges per node of a 4-connected label map (twice that for a 6-connected volume)
+EDGE_CAP_PER_NODE = 8
 #: edge_type -> (metric, spatial) of isb_gc_energies; only 'model' and 'spatial' are spatially normalised
 #: (reference graph_cuts.py:646)
 EDGE_MODES = {'': (0, 0), 'model': (1, 1), 'model_lT': (1, 0), 'model_l1': (2, 0), 'model_l2': (3, 0), 'spatial': (0, 1)}
+
+
+def flag_bits(flags):
+    """(bit mask, number of statistics) of a list of FLAG_BITS names"""
+    bits = 0
+    for f in flags:
+        bits |= FLAG_BITS[f]
+    return bits, bin(bits).count('1')
+
+
+def dtype_code(dtype):
+    """C-ABI element type code of a numpy or torch dtype"""
+    name = str(dtype)
+    return _lib.DTYPE_CODES[name[len('torch.'):] if name.startswith('torch.') else np.dtype(dtype).name]
+
+
+def edge_capacity(nodes, ndim=2):
+    """rows of a device edge table over ``nodes`` labels of a ``ndim``-D label map, first attempt: EDGE_CAP_PER_NODE per node
+    (twice as many in 3-D)"""
+    return max(64, EDGE_CAP_PER_NODE * (ndim - 1) * int(nodes))
+
+
+def grown_edge_capacity(cap):
+    """rows of the next attempt after a table of ``cap`` rows overflowed.  An overflowed table reports cap + 1 edges and no
+    kernel reads it, so the retry computes the same whatever the growth factor."""
+    return 4 * int(cap)
 
 
 def gaussian_half_kernel(sigma, truncate=4.0):
@@ -73,6 +102,25 @@ class Engine(object):
         self.lib = _lib.lib()
         self.device = self.torch.device('cuda', self.torch.cuda.current_device() if device is None else device)
         self._bufs = {}
+        self._fns = {name[len('isb_'):]: getattr(self.lib, name) for name in _lib.SIGNATURES}
+
+    # -- C-ABI calls -----------------------------------------------------------------------------------------------
+    def call(self, name, *args):
+        """``isb_<name>(*args, stream)`` on the CURRENT stream (read at every call: graph capture and the side stream switch it),
+        raising on an error status.  A torch tensor passes as its device pointer, a (float64) numpy array as a pointer to its
+        data, anything else as it is (the argtypes of ``_lib.SIGNATURES`` convert numbers and take a struct by reference)."""
+        tensor = self.torch.Tensor
+        _lib.check(self._fns[name](*[a.data_ptr() if isinstance(a, tensor) else a.ctypes.data_as(_DOUBLE_P) if isinstance(a, np.ndarray)
+                                     else a for a in args], self.torch.cuda.current_stream().cuda_stream))
+
+    def query(self, name, *args):
+        """value of the host-side C-ABI function ``isb_<name>(*args)`` (workspace sizes, launch counter)"""
+        return self._fns[name](*args)
+
+    def workspace(self, name, query, *args):
+        """cached byte buffer ``name`` of the size ``isb_<query>(*args)`` asks for; returns (buffer, bytes)"""
+        wsb = self._fns[query](*args)
+        return self.buf(name, (wsb,), self.torch.uint8), wsb
 
     # -- memory helpers ------------------------------------------------------------------------------------------
     def buf(self, name, shape, dtype):
@@ -177,108 +225,100 @@ class Engine(object):
             self.torch.cuda.current_stream().synchronize()
         return out.numpy()
 
+    def download(self, tensors):
+        """copies of device tensors into pinned host tensors, queued on the current stream; returns (host tensors, an event recorded
+        after the copies) -- the caller synchronises on the event when it needs the data"""
+        hosts = []
+        for t in tensors:
+            h = self.pinned_empty(t.shape, t.dtype)
+            h.copy_(t, non_blocking=True)
+            hosts.append(h)
+        event = self.torch.cuda.Event()
+        event.record()
+        return hosts, event
+
     def side_stream(self):
         """a second CUDA stream of this engine (copies that may overlap the kernels of the main stream)"""
         if getattr(self, '_side', None) is None:
             self._side = self.torch.cuda.Stream(device=self.device)
         return self._side
 
-    def _ck(self, rc):
-        _lib.check(rc)
-
     # -- (i) SLIC -------------------------------------------------------------------------------------------------
+    @staticmethod
+    def slic_setup(H, W, n_segments, sigma):
+        """host-side set-up of the whole-image and the banded SLIC: (half Gaussian kernel, its radius, seed grid [n, 2], step_y,
+        step_x, step)"""
+        w_half, radius = gaussian_half_kernel(sigma) if sigma > 0 else (np.ones(1), 0)
+        seeds, ty, tx = slic_seed_grid(H, W, n_segments)
+        return w_half, radius, seeds, ty, tx, float(max(1, ty, tx))
+
+    def connectivity(self, km, n_segments, min_size_factor=0.5, max_size_factor=3):
+        """connectivity pass over a k-means label map [H, W]; returns (labels int32 [H, W], n_labels device int32[1])"""
+        H, W = int(km.shape[0]), int(km.shape[1])
+        segment_size = H * W / n_segments
+        min_size, max_size = int(min_size_factor * segment_size), int(max_size_factor * segment_size)
+        cws, cwsb = self.workspace('ws_conn', 'connectivity_workspace_bytes', H, W)
+        out = self.buf('labels', (H, W), self.torch.int32)
+        n_labels = self.buf('n_labels', (1,), self.torch.int32)
+        self.call('enforce_connectivity', km, H, W, min_size, max_size, out, n_labels, cws, cwsb)
+        return out, n_labels
+
     def slic(self, d_img, n_segments, compactness, sigma=1.0, max_iter=10, enforce_connectivity=True,
              min_size_factor=0.5, max_size_factor=3, slic_zero=False, rescale=True):
         """device SLIC on a [H,W,C] device tensor; returns (labels int32 [H,W] device, n_labels device int32[1] or None)"""
-        torch, lib = self.torch, self.lib
+        torch = self.torch
         H, W = int(d_img.shape[0]), int(d_img.shape[1])
         Cn = 1 if d_img.dim() == 2 else int(d_img.shape[2])
-        code = _lib.DTYPE_CODES[str(d_img.dtype).replace('torch.', '')]
-        st = _lib.stream_ptr()
+        w_half, radius, seeds, ty, tx, step = self.slic_setup(H, W, n_segments, sigma)
         lab = self.buf('lab', (3, H, W), torch.float64)
         mm = self.buf('minmax', (4,), torch.float64)
-        if sigma > 0:
-            w_half, radius = gaussian_half_kernel(sigma)
-        else:
-            w_half, radius = np.ones(1), 0
-        self._ck(lib.isb_slic_prepare(_lib.ptr(d_img), code, H, W, Cn, w_half.ctypes.data_as(C.POINTER(C.c_double)), radius,
-                                      C.c_double(1.0 / compactness), int(bool(rescale)), _lib.ptr(lab), _lib.ptr(mm), st))
-        seeds, ty, tx = slic_seed_grid(H, W, n_segments)
+        self.call('slic_prepare', d_img, dtype_code(d_img.dtype), H, W, Cn, w_half, radius, 1.0 / compactness, int(bool(rescale)), lab, mm)
         n_seeds = len(seeds)
-        step = float(max(1, ty, tx))
         d_seeds = self.const_device(seeds, 'seeds')
-        wsb = lib.isb_slic_kmeans_workspace_bytes(H, W, n_seeds, ty, tx)
-        ws = self.buf('ws_kmeans', (wsb,), torch.uint8)
+        ws, wsb = self.workspace('ws_kmeans', 'slic_kmeans_workspace_bytes', H, W, n_seeds, ty, tx)
         km = self.buf('labels_km', (H, W), torch.int32)
-        self._ck(lib.isb_slic_kmeans(_lib.ptr(lab), H, W, _lib.ptr(d_seeds), n_seeds, ty, tx, C.c_double(step), int(max_iter),
-                                     int(bool(slic_zero)), _lib.ptr(km), None, _lib.ptr(ws), C.c_size_t(wsb), st))
+        self.call('slic_kmeans', lab, H, W, d_seeds, n_seeds, ty, tx, step, int(max_iter), int(bool(slic_zero)), km, None, ws, wsb)
         if not enforce_connectivity:
             return km, None
-        segment_size = 1 * H * W / n_segments
-        min_size, max_size = int(min_size_factor * segment_size), int(max_size_factor * segment_size)
-        cwsb = lib.isb_connectivity_workspace_bytes(H, W)
-        cws = self.buf('ws_conn', (cwsb,), torch.uint8)
-        out = self.buf('labels', (H, W), torch.int32)
-        n_labels = self.buf('n_labels', (1,), torch.int32)
-        self._ck(lib.isb_enforce_connectivity(_lib.ptr(km), H, W, min_size, max_size, _lib.ptr(out), _lib.ptr(n_labels),
-                                              _lib.ptr(cws), C.c_size_t(cwsb), st))
-        return out, n_labels
+        return self.connectivity(km, n_segments, min_size_factor, max_size_factor)
 
     def slic3d(self, d_vol, n_segments, compactness, spacing=(1, 1, 1), sigma=1.0, max_iter=10, enforce_connectivity=True,
                min_size_factor=0.5, max_size_factor=3):
         """device SLIC of a single-channel volume [D, H, W] (csrc/slic3d.cu); returns (labels int32 [D,H,W], n_labels or None)"""
-        torch, lib = self.torch, self.lib
+        torch = self.torch
         D, H, W = (int(v) for v in d_vol.shape)
-        code = _lib.DTYPE_CODES[str(d_vol.dtype).replace('torch.', '')]
-        st = _lib.stream_ptr()
         spacing = np.ascontiguousarray(spacing, dtype=np.float64)
         halves = []
         for axis, sig in enumerate(np.array([sigma, sigma, sigma], dtype=np.float64) / spacing):
             w_half, radius = gaussian_half_kernel(sig) if sigma > 0 else (np.ones(1), 0)
-            halves.append((self.to_device(w_half, 'slic3d_w%d' % axis), radius))
+            halves += [self.to_device(w_half, 'slic3d_w%d' % axis), radius]
         tmp = self.buf('slic3d_tmp', (D, H, W), torch.float64)
         scaled = self.buf('slic3d_vol', (D, H, W), torch.float64)
-        self._ck(lib.isb_slic3d_prepare(_lib.ptr(d_vol), code, D, H, W, _lib.ptr(halves[0][0]), halves[0][1], _lib.ptr(halves[1][0]),
-                                        halves[1][1], _lib.ptr(halves[2][0]), halves[2][1], C.c_double(1.0 / compactness), _lib.ptr(tmp),
-                                        _lib.ptr(scaled), st))
+        self.call('slic3d_prepare', d_vol, dtype_code(d_vol.dtype), D, H, W, *halves, 1.0 / compactness, tmp, scaled)
         seeds, steps = slic_seed_grid3d((D, H, W), n_segments)
         n_seeds = len(seeds)
         d_seeds = self.to_device(seeds, 'seeds3d')
-        wsb = lib.isb_slic3d_kmeans_workspace_bytes(D, H, W, n_seeds)
-        ws = self.buf('ws_kmeans3d', (wsb,), torch.uint8)
+        ws, wsb = self.workspace('ws_kmeans3d', 'slic3d_kmeans_workspace_bytes', D, H, W, n_seeds)
         km = self.buf('labels_km3d', (D, H, W), torch.int32)
-        self._ck(lib.isb_slic3d_kmeans(_lib.ptr(scaled), D, H, W, _lib.ptr(d_seeds), n_seeds, steps[0], steps[1], steps[2],
-                                       C.c_double(float(max(steps))), spacing.ctypes.data_as(C.POINTER(C.c_double)), int(max_iter),
-                                       _lib.ptr(km), _lib.ptr(ws), C.c_size_t(wsb), st))
+        self.call('slic3d_kmeans', scaled, D, H, W, d_seeds, n_seeds, steps[0], steps[1], steps[2], float(max(steps)), spacing,
+                  int(max_iter), km, ws, wsb)
         if not enforce_connectivity:
             return km, None
         segment_size = D * H * W / n_segments
         min_size, max_size = int(min_size_factor * segment_size), int(max_size_factor * segment_size)
-        cwsb = lib.isb_connectivity3d_workspace_bytes(D, H, W, max(max_size, 1))
-        cws = self.buf('ws_conn3d', (cwsb,), torch.uint8)
+        cws, cwsb = self.workspace('ws_conn3d', 'connectivity3d_workspace_bytes', D, H, W, max(max_size, 1))
         out = self.buf('labels3d', (D, H, W), torch.int32)
         n_labels = self.buf('n_labels', (1,), torch.int32)
-        self._ck(lib.isb_enforce_connectivity3d(_lib.ptr(km), D, H, W, min_size, max_size, _lib.ptr(out), _lib.ptr(n_labels), _lib.ptr(cws),
-                                                C.c_size_t(cwsb), st))
+        self.call('enforce_connectivity3d', km, D, H, W, min_size, max_size, out, n_labels, cws, cwsb)
         return out, n_labels
 
-    def graph3d(self, d_seg, nb, cap=None):
-        """6-connected label pairs and centres (z, y, x) of a device label volume: (edges [cap,2], n_edges dev, cap, centres [nb,3])"""
-        torch, lib = self.torch, self.lib
-        D, H, W = (int(v) for v in d_seg.shape)
-        if cap is None:
-            cap = max(64, 16 * int(nb))
-        wsb = lib.isb_adjacency_workspace_bytes(int(nb), int(cap))
-        ws = self.buf('ws_adj', (wsb,), torch.uint8)
-        edges = self.buf('edges', (cap, 2), torch.int32)
-        n_edges = self.buf('n_edges', (1,), torch.int32)
-        self._ck(lib.isb_adjacency_edges_3d(_lib.ptr(d_seg), D, H, W, int(nb), _lib.ptr(edges), int(cap), _lib.ptr(n_edges), _lib.ptr(ws),
-                                            C.c_size_t(wsb), _lib.stream_ptr()))
-        centres = self.buf('centres3d', (nb, 3), torch.float64)
-        cws = self.buf('ws_centres3d', (4 * int(nb),), torch.int64)
-        self._ck(lib.isb_centroids_3d(_lib.ptr(d_seg), D, H, W, int(nb), _lib.ptr(centres), _lib.ptr(cws), C.c_size_t(32 * int(nb)),
-                                      _lib.stream_ptr()))
-        return edges, n_edges, cap, centres
+    def centroids3d(self, d_seg, nb):
+        """centres (z, y, x) [nb, 3] of the labels of a device label volume"""
+        nb = int(nb)
+        centres = self.buf('centres3d', (nb, 3), self.torch.float64)
+        cws = self.buf('ws_centres3d', (4 * nb,), self.torch.int64)
+        self.call('centroids_3d', d_seg, *d_seg.shape, nb, centres, cws, 32 * nb)
+        return centres
 
     def slic_label_bound(self, H, W, n_segments, min_size_factor=0.5):
         """upper bound on the number of labels after connectivity enforcement (each kept label has >= min_size px)"""
@@ -288,99 +328,97 @@ class Engine(object):
     # -- (ii) descriptors -----------------------------------------------------------------------------------------
     def segment_stats(self, d_img, d_seg, nb, flags, feat=None, col0=0, want_centres=False, want_counts=False):
         """colour statistics (+centroids) of a [H,W,3] device image over labels [H,W] int32 in [0, nb)"""
-        torch, lib = self.torch, self.lib
+        torch = self.torch
         H, W = int(d_seg.shape[0]), int(d_seg.shape[1])
-        code = 0 if d_img is None else _lib.DTYPE_CODES[str(d_img.dtype).replace('torch.', '')]
-        bits = 0
-        for f in flags:
-            bits |= FLAG_BITS[f]
-        ncol = 3 * bin(bits).count('1')
-        if feat is None and ncol:
-            feat = self.buf('feat', (nb, ncol), torch.float64)
+        nb = int(nb)
+        bits, n = flag_bits(flags)
+        if feat is None and n:
+            feat = self.buf('feat', (nb, 3 * n), torch.float64)
         ld = int(feat.shape[1]) if feat is not None else 0
         centres = self.buf('centres', (nb, 2), torch.float64) if want_centres else None
         counts = self.buf('counts', (nb,), torch.int32) if want_counts else None
-        wsb = lib.isb_segment_stats_workspace_bytes(nb)
-        ws = self.buf('ws_stats', (wsb,), torch.uint8)
-        self._ck(lib.isb_segment_stats_2d(_lib.ptr(d_img), code, _lib.ptr(d_seg), H, W, int(nb), bits, _lib.ptr(feat), ld, int(col0),
-                                          _lib.ptr(centres), _lib.ptr(counts), _lib.ptr(ws), C.c_size_t(wsb), _lib.stream_ptr()))
+        ws, wsb = self.workspace('ws_stats', 'segment_stats_workspace_bytes', nb)
+        self.call('segment_stats_2d', d_img, 0 if d_img is None else dtype_code(d_img.dtype), d_seg, H, W, nb, bits, feat, ld, int(col0),
+                  centres, counts, ws, wsb)
         return feat, centres, counts
 
     # -- (iii) graph, energies, alpha-expansion ---------------------------------------------------------------------
     def adjacency(self, d_seg, nb, cap=None):
-        """unique 4-connected label pairs; returns (edges int32 [cap,2] device, n_edges device int32[1], cap)"""
-        torch, lib = self.torch, self.lib
-        H, W = int(d_seg.shape[0]), int(d_seg.shape[1])
-        if cap is None:
-            cap = max(64, 8 * int(nb))
-        wsb = lib.isb_adjacency_workspace_bytes(int(nb), int(cap))
-        ws = self.buf('ws_adj', (wsb,), torch.uint8)
+        """unique 4-connected (6-connected in a volume) label pairs of a device label map;
+        returns (edges int32 [cap,2] device, n_edges device int32[1], cap)"""
+        torch = self.torch
+        nb = int(nb)
+        cap = edge_capacity(nb, d_seg.dim()) if cap is None else int(cap)
+        ws, wsb = self.workspace('ws_adj', 'adjacency_workspace_bytes', nb, cap)
         edges = self.buf('edges', (cap, 2), torch.int32)
         n_edges = self.buf('n_edges', (1,), torch.int32)
-        self._ck(lib.isb_adjacency_edges(_lib.ptr(d_seg), H, W, int(nb), _lib.ptr(edges), int(cap), _lib.ptr(n_edges), _lib.ptr(ws),
-                                         C.c_size_t(wsb), _lib.stream_ptr()))
+        self.call('adjacency_edges' if d_seg.dim() == 2 else 'adjacency_edges_3d', d_seg, *d_seg.shape, nb, edges, cap, n_edges, ws, wsb)
         return edges, n_edges, cap
 
     def gc_energies(self, d_proba, d_edges, E, d_n_edges, d_centres, edge_mode, edge_cost, pairwise, d_n_nodes=None):
-        torch, lib = self.torch, self.lib
-        N, K = int(d_proba.shape[0]), int(d_proba.shape[1])
+        torch = self.torch
+        N, K, E = int(d_proba.shape[0]), int(d_proba.shape[1]), int(E)
         d_pw = self.const_device(np.ascontiguousarray(pairwise, dtype=np.float64), 'pairwise')
         unary = self.buf('unary', (N, K), torch.float64)
         edge_w = self.buf('edge_w', (max(E, 1),), torch.float64)
         unary_i = self.buf('unary_i', (N, K), torch.int32)
         edge_wi = self.buf('edge_wi', (max(E, 1),), torch.int32)
         smooth_i = self.buf('smooth_i', (K, K), torch.int32)
-        wsb = lib.isb_gc_energies_workspace_bytes(N, K, int(E))
-        ws = self.buf('ws_energy', (wsb,), torch.uint8)
-        self._ck(lib.isb_gc_energies(_lib.ptr(d_proba), N, _lib.ptr(d_n_nodes), K, _lib.ptr(d_edges), int(E), _lib.ptr(d_n_edges), _lib.ptr(d_centres),
-                                     int(edge_mode[0]), int(edge_mode[1]), C.c_double(edge_cost), _lib.ptr(d_pw), _lib.ptr(unary), _lib.ptr(edge_w),
-                                     _lib.ptr(unary_i), _lib.ptr(edge_wi), _lib.ptr(smooth_i), _lib.ptr(ws), C.c_size_t(wsb),
-                                     _lib.stream_ptr()))
+        ws, wsb = self.workspace('ws_energy', 'gc_energies_workspace_bytes', N, K, E)
+        self.call('gc_energies', d_proba, N, d_n_nodes, K, d_edges, E, d_n_edges, d_centres, int(edge_mode[0]), int(edge_mode[1]),
+                  float(edge_cost), d_pw, unary, edge_w, unary_i, edge_wi, smooth_i, ws, wsb)
         return unary, edge_w, unary_i, edge_wi, smooth_i
 
     def alpha_expansion(self, N, K, E, d_n_edges, d_edges, edge_wi, unary_i, smooth_i, n_iter=-1, init_labels=None,
                         d_n_nodes=None):
-        torch, lib = self.torch, self.lib
+        torch = self.torch
+        N, K, E = int(N), int(K), int(E)
         labels = self.buf('gc_labels', (N,), torch.int32)
         if init_labels is None:
-            self._ck(lib.isb_fill_i32(_lib.ptr(labels), C.c_longlong(int(N)), 0, _lib.stream_ptr()))
+            self.call('fill_i32', labels, N, 0)
         else:
             labels.copy_(init_labels)  # device-to-device memcpy of a caller-supplied labeling
         energy = self.buf('gc_energy', (1,), torch.int64)
         stats = self.buf('gc_stats', (8,), torch.int32)
-        wsb = lib.isb_alpha_expansion_workspace_bytes(int(N), int(K), int(E))
-        ws = self.buf('ws_gc', (wsb,), torch.uint8)
-        self._ck(lib.isb_alpha_expansion(int(N), _lib.ptr(d_n_nodes), int(K), int(E), _lib.ptr(d_n_edges), _lib.ptr(d_edges), _lib.ptr(edge_wi),
-                                         _lib.ptr(unary_i), _lib.ptr(smooth_i), int(n_iter), _lib.ptr(labels), _lib.ptr(energy),
-                                         _lib.ptr(stats), _lib.ptr(ws), C.c_size_t(wsb), _lib.stream_ptr()))
+        ws, wsb = self.workspace('ws_gc', 'alpha_expansion_workspace_bytes', N, K, E)
+        self.call('alpha_expansion', N, d_n_nodes, K, E, d_n_edges, d_edges, edge_wi, unary_i, smooth_i, int(n_iter), labels, energy,
+                  stats, ws, wsb)
         return labels, energy, stats
+
+    def graph_cut(self, d_proba, d_edges, E, d_n_edges, d_centres, edge_mode, edge_cost, pairwise, d_n_nodes=None):
+        """energies of the superpixel graph [N = d_proba rows, K classes] and the alpha-expansion over them (asynchronous);
+        returns (labels [N] int32, unary [N, K], edge weights [E]) on the device"""
+        unary, edge_w, unary_i, edge_wi, smooth_i = self.gc_energies(d_proba, d_edges, E, d_n_edges, d_centres, edge_mode, edge_cost,
+                                                                     pairwise, d_n_nodes=d_n_nodes)
+        labels, _, _ = self.alpha_expansion(d_proba.shape[0], d_proba.shape[1], E, d_n_edges, d_edges, edge_wi, unary_i, smooth_i, -1,
+                                            d_n_nodes=d_n_nodes)
+        return labels, unary, edge_w
 
     def gmm_fit_predict(self, d_feat, K, n_init, max_iter, use_scaler=True, seed=0, d_n=None, init_labels=None, tol=1e-3,
                         reg_covar=1e-6):
         """device class model: returns (proba [N,K] device, params device vector; see isb_gmm_fit_predict)"""
-        torch, lib = self.torch, self.lib
-        N, D = int(d_feat.shape[0]), int(d_feat.shape[1])
+        torch = self.torch
+        N, D, K, n_init = int(d_feat.shape[0]), int(d_feat.shape[1]), int(K), int(n_init)
         ld = int(d_feat.stride(0))
         proba = self.buf('proba', (N, K), torch.float64)
-        params = self.buf('gmm_params', (lib.isb_gmm_params_len(D, K),), torch.float64)
-        wsb = lib.isb_gmm_workspace_bytes(N, D, int(K), int(n_init))
-        ws = self.buf('ws_gmm', (wsb,), torch.uint8)
+        params = self.buf('gmm_params', (self.query('gmm_params_len', D, K),), torch.float64)
+        ws, wsb = self.workspace('ws_gmm', 'gmm_workspace_bytes', N, D, K, n_init)
         d_init = None
         if init_labels is not None:
             d_init = self.to_device(np.ascontiguousarray(init_labels, dtype=np.int32), 'gmm_init')
-        self._ck(lib.isb_gmm_fit_predict(_lib.ptr(d_feat), N, D, ld, _lib.ptr(d_n), int(K), int(n_init), int(max_iter), C.c_double(tol),
-                                         C.c_double(reg_covar), int(bool(use_scaler)), C.c_ulonglong(int(seed)), _lib.ptr(d_init),
-                                         _lib.ptr(proba), _lib.ptr(params), _lib.ptr(ws), C.c_size_t(wsb), _lib.stream_ptr()))
+        self.call('gmm_fit_predict', d_feat, N, D, ld, d_n, K, n_init, int(max_iter), float(tol), float(reg_covar), int(bool(use_scaler)),
+                  int(seed), d_init, proba, params, ws, wsb)
         return proba, params
 
-    def gather(self, d_seg, lut_i=None, lut_p=None):
-        torch, lib = self.torch, self.lib
+    def gather(self, d_seg, lut_i=None, lut_p=None, out_i=None):
+        """segm = lut_i[seg] (into ``out_i`` or the cached 'segm') and segm_soft = lut_p[seg] over a device label map [H, W]"""
+        torch = self.torch
         H, W = int(d_seg.shape[0]), int(d_seg.shape[1])
-        out_i = self.buf('segm', (H, W), torch.int32) if lut_i is not None else None
+        if out_i is None and lut_i is not None:
+            out_i = self.buf('segm', (H, W), torch.int32)
         K = int(lut_p.shape[1]) if lut_p is not None else 0
         out_p = self.buf('segm_soft', (H, W, K), torch.float64) if lut_p is not None else None
-        self._ck(lib.isb_gather(_lib.ptr(d_seg), C.c_longlong(H * W), _lib.ptr(lut_i), _lib.ptr(lut_p), K, _lib.ptr(out_i),
-                                _lib.ptr(out_p), _lib.stream_ptr()))
+        self.call('gather', d_seg, H * W, lut_i, lut_p, K, out_i, out_p)
         return out_i, out_p
 
 

@@ -393,13 +393,8 @@ def _edge_weights_volume(eng, segments, proba, edge_type):
     _edge_mode(edge_type)     # validates the name
     nb = int(segments.max()) + 1
     d_seg = eng.to_device(segments.astype(np.int32, copy=False), 'seg_in3d')
-    cap = None
-    while True:
-        d_edges, d_n, cap, d_centres = eng.graph3d(d_seg, nb, cap)
-        E = int(eng.to_host(d_n)[0])
-        if E <= cap:
-            break
-        cap = 2 * E
+    d_edges, E = device_adjacency(eng, d_seg, nb)
+    d_centres = eng.centroids3d(d_seg, nb)
     edges = eng.to_host(d_edges[:E]).copy() if E else np.zeros((0, 2), dtype=np.int32)
     if not E:
         return edges, np.zeros(0)
@@ -451,9 +446,7 @@ def segment_graph_cut_general(segments, proba, image=None, features=None, gc_reg
         centres = None
         if mode[1]:
             _, centres, _ = eng.segment_stats(None, d_seg, nb, (), want_centres=True)
-        unary, edge_w, unary_i, edge_wi, smooth_i = eng.gc_energies(d_proba, d_edges, E, None, centres, mode, float(edge_cost),
-                                                                    pairwise_cost)
-        labels, _, _ = eng.alpha_expansion(len(proba), proba.shape[1], E, None, d_edges, edge_wi, unary_i, smooth_i, -1)
+        labels, unary, edge_w = eng.graph_cut(d_proba, d_edges, E, None, centres, mode, float(edge_cost), pairwise_cost)
         graph_labels = eng.to_host(labels).copy()
         if debug_visual is not None:
             edges, edge_weights = eng.to_host(d_edges[:E]).copy(), eng.to_host(edge_w[:E]).copy()

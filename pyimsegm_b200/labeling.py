@@ -4,7 +4,6 @@ pipeline calls per image: ``wrapper_compute_color2d_slic_features_labels``, refe
 """
 import numpy as np
 
-from . import _lib
 from .engine import get_engine
 from .utilities import ImageDimensionError
 
@@ -29,8 +28,7 @@ def histogram_regions_labels_counts(slic, segm):
     d_a = eng.to_device(slic.astype(np.int32, copy=False), 'hist_slic')
     d_b = eng.to_device(segm.astype(np.int32, copy=False), 'hist_annot')
     hist = eng.buf('hist_joint', (nb_a, nb_b), eng.torch.int32)
-    _lib.check(eng.lib.isb_region_label_hist(_lib.ptr(d_a), _lib.ptr(d_b), slic.shape[0], slic.shape[1], nb_a, nb_b, _lib.ptr(hist),
-                                             _lib.stream_ptr()))
+    eng.call('region_label_hist', d_a, d_b, slic.shape[0], slic.shape[1], nb_a, nb_b, hist)
     return eng.to_host(hist).astype(float)
 
 

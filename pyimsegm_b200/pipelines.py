@@ -18,7 +18,7 @@ import logging
 import numpy as np
 
 from .descriptors import FEATURES_SET_COLOR, compute_selected_features_img2d, flags_are_native, native_feature_layout
-from .engine import get_engine
+from .engine import edge_capacity, get_engine, grown_edge_capacity
 from .graph_cuts import (_edge_mode, compute_pairwise_cost, device_gmm_applicable, estim_class_model,
                          segment_graph_cut_general)
 from .superpixels import _as_rgb_like, _supported_dtype, slic_params
@@ -97,18 +97,32 @@ def compute_color2d_superpixels_features(image, dict_features, sp_size=30, sp_re
     return slic, features
 
 
-def _device_graphcut(eng, res, nb, d_proba, K, gc_regul, gc_edge_type, d_n_nodes=None, want_soft=True, edge_cap=None):
+def _device_graphcut(eng, res, nb, d_proba, gc_regul, gc_edge_type, d_n_nodes=None, want_soft=True, edge_cap=None, rows=None,
+                     whole_segm=False):
     """device tail of the pipeline: adjacency, energies, alpha-expansion, LUT gathers (all asynchronous).
-    ``nb`` may be an upper bound of the label count when ``d_n_nodes`` (device scalar) carries the real one.
+    ``nb`` (= the rows of ``d_proba``) may be an upper bound of the label count when ``d_n_nodes`` (device scalar) carries the real
+    one.  ``rows`` = (lo, hi): gather only these rows of the label map, into rows lo:hi of a whole-image 'segm' when ``whole_segm``.
     Returns (d_labels, d_segm, d_soft, d_n_edges, edge_cap)."""
-    pairwise = compute_pairwise_cost(gc_regul, (nb, K))
+    pairwise = compute_pairwise_cost(gc_regul, d_proba.shape)
     d_edges, d_n_edges, edge_cap = eng.adjacency(res.d_seg, nb, edge_cap)
-    mode = _edge_mode(gc_edge_type)
-    _, _, unary_i, edge_wi, smooth_i = eng.gc_energies(d_proba, d_edges, edge_cap, d_n_edges, res.d_centres, mode, 1.0, pairwise,
-                                                       d_n_nodes=d_n_nodes)
-    d_labels, _, _ = eng.alpha_expansion(nb, K, edge_cap, d_n_edges, d_edges, edge_wi, unary_i, smooth_i, -1, d_n_nodes=d_n_nodes)
-    d_segm, d_soft = eng.gather(res.d_seg, d_labels, d_proba if want_soft else None)
+    d_labels, _, _ = eng.graph_cut(d_proba, d_edges, edge_cap, d_n_edges, res.d_centres, _edge_mode(gc_edge_type), 1.0, pairwise,
+                                   d_n_nodes=d_n_nodes)
+    d_seg = res.d_seg if rows is None else res.d_seg[rows[0]:rows[1]]
+    out_segm = eng.buf('segm', res.d_seg.shape, eng.torch.int32)[rows[0]:rows[1]] if whole_segm else None
+    d_segm, d_soft = eng.gather(d_seg, d_labels, d_proba if want_soft else None, out_i=out_segm)
     return d_labels, d_segm, d_soft, d_n_edges, edge_cap
+
+
+def _soft_on_side_stream(eng, d_seg, d_proba):
+    """segm_soft = proba[d_seg] needs only the class probabilities: its gather and its (large) download run on the engine's side
+    stream while the main stream builds and cuts the graph.  Returns (pinned host tensor, event of the download)."""
+    torch = eng.torch
+    side = eng.side_stream()
+    side.wait_stream(torch.cuda.current_stream())
+    with torch.cuda.stream(side):
+        _, d_soft = eng.gather(d_seg, None, d_proba)
+        (host, ), event = eng.download([d_soft])
+    return host, event
 
 
 def _argmin_labels_device(eng, proba):
@@ -118,10 +132,6 @@ def _argmin_labels_device(eng, proba):
 
 #: start the download of segm_soft (it only needs the class probabilities) on a side stream while the graph is cut
 EARLY_SOFT_DOWNLOAD = True
-
-#: initial capacity of the device edge table, in edges per (upper bound of) superpixel; grown x4 on overflow
-EDGE_CAP_PER_NODE = [8]
-
 
 #: replay the device part of the path as CUDA graphs once a configuration has been seen twice (the ~70 kernel launches of an image
 #: cost more host time than the GPU needs for them when images are processed back to back, and the gaps between them add up)
@@ -142,7 +152,7 @@ def _graph_call(eng, key, fn):
     torch = eng.torch
     if entry == 'seen':
         graph = torch.cuda.CUDAGraph()
-        n0 = eng.lib.isb_launch_count()
+        n0 = eng.query('launch_count')
         cur = torch.cuda.current_stream()
         side = torch.cuda.Stream(device=eng.device)
         side.wait_stream(cur)
@@ -150,10 +160,10 @@ def _graph_call(eng, key, fn):
             out = fn()
         cur.wait_stream(side)
         eng.graphs_captured = getattr(eng, 'graphs_captured', 0) + 1      # from now on the engine never frees a buffer it outgrows
-        entry = _GRAPHS[key] = (graph, out, int(eng.lib.isb_launch_count() - n0))
+        entry = _GRAPHS[key] = (graph, out, int(eng.query('launch_count') - n0))
     graph, out, n_kernels = entry
     graph.replay()
-    eng.lib.isb_note_graph_replay(n_kernels)
+    eng.query('note_graph_replay', n_kernels)
     return out
 
 
@@ -161,7 +171,7 @@ def _features_key(dict_features):
     return tuple(sorted((k, tuple(v)) for k, v in dict_features.items()))
 
 
-def _run_resident(eng, image, model, dict_features, sp_size, sp_regul, gc_regul, gc_edge_type, soft_sink=None):
+def _run_resident(eng, image, model, dict_features, sp_size, sp_regul, gc_regul, gc_edge_type, soft_sink=None, edge_cap=None):
     """the whole hot path on the device.  ``model`` is either ('fit', nb_classes, use_scaler, max_iter) -> the default
     GMM is fitted on the GPU and NOTHING syncs with the host until the results are ready; or a callable
     proba_fn(features) -> one round trip (features down, probabilities up) as in the reference.
@@ -169,6 +179,7 @@ def _run_resident(eng, image, model, dict_features, sp_size, sp_regul, gc_regul,
     (it does not depend on the graph cut) -- then ``d_soft`` is returned as None.
     With a device-fitted model and colour features the two halves -- image -> class probabilities, probabilities -> cut and LUT
     gathers -- are CUDA-graph replays (:func:`_graph_call`); the image then has to sit in one of the engine's cached buffers.
+    ``edge_cap``: capacity of the edge table (default :func:`engine.edge_capacity` of the superpixel count).
     Returns (d_segm, d_soft, check): ``check`` is None or (d_n_edges, edge_cap) still to be verified by the caller."""
     no_cut = (not isinstance(gc_regul, (list, np.ndarray))) and gc_regul <= 0
     if isinstance(model, tuple):
@@ -193,12 +204,12 @@ def _run_resident(eng, image, model, dict_features, sp_size, sp_regul, gc_regul,
             nb = int(eng.to_host(res.d_n_labels)[0])
             d_labels = _argmin_labels_device(eng, eng.to_host(d_proba[:nb]))
             return eng.gather(res.d_seg, d_labels, d_proba) + (None, )
-        cap = max(64, EDGE_CAP_PER_NODE[0] * res.nb_bound)
+        cap = edge_cap or edge_capacity(res.nb_bound)
         if soft_sink is not None:
             soft_sink(res.d_seg, d_proba)
 
         def second_half():
-            return _device_graphcut(eng, res, res.nb_bound, d_proba, nb_classes, gc_regul, gc_edge_type, d_n_nodes=res.d_n_labels,
+            return _device_graphcut(eng, res, res.nb_bound, d_proba, gc_regul, gc_edge_type, d_n_nodes=res.d_n_labels,
                                     want_soft=soft_sink is None, edge_cap=cap)
 
         key2 = ('cut', id(eng), res.d_seg.data_ptr(), d_proba.data_ptr(), res.d_centres.data_ptr(), res.shape, res.nb_bound, nb_classes,
@@ -214,26 +225,22 @@ def _run_resident(eng, image, model, dict_features, sp_size, sp_regul, gc_regul,
     d_proba = eng.to_device(proba, 'proba')
     if no_cut:
         return eng.gather(res.d_seg, _argmin_labels_device(eng, proba), d_proba) + (None, )
-    cap = max(64, EDGE_CAP_PER_NODE[0] * nb)
+    cap = edge_cap or edge_capacity(nb)
     if soft_sink is not None:
         soft_sink(res.d_seg, d_proba)
-    _, d_segm, d_soft, d_n_edges, cap = _device_graphcut(eng, res, nb, d_proba, proba.shape[1], gc_regul, gc_edge_type,
-                                                         want_soft=soft_sink is None, edge_cap=cap)
+    _, d_segm, d_soft, d_n_edges, cap = _device_graphcut(eng, res, nb, d_proba, gc_regul, gc_edge_type, want_soft=soft_sink is None,
+                                                         edge_cap=cap)
     return d_segm, d_soft, (d_n_edges, cap)
 
 
 def _download_results(eng, tensors):
     """D2H into pinned buffers with ONE synchronisation; returns numpy views"""
-    outs = []
-    for t in tensors:
-        h = eng.pinned_empty(t.shape, t.dtype)
-        h.copy_(t, non_blocking=True)
-        outs.append(h)
-    eng.torch.cuda.current_stream().synchronize()
-    return [h.numpy() for h in outs]
+    hosts, event = eng.download(tensors)
+    event.synchronize()
+    return [h.numpy() for h in hosts]
 
 
-def _segment(image, model, dict_features, sp_size, sp_regul, gc_regul, gc_edge_type, debug_visual, classes=None):
+def _segment(image, model, dict_features, sp_size, sp_regul, gc_regul, gc_edge_type, debug_visual, classes=None, edge_cap=None):
     image = np.asarray(image)
     eng = get_engine()
     native = image.ndim == 3 and flags_are_native(dict_features) and gc_edge_type not in ('color', 'features')
@@ -253,42 +260,28 @@ def _segment(image, model, dict_features, sp_size, sp_regul, gc_regul, gc_edge_t
         if classes is not None:
             graph_labels = classes[graph_labels]
         return graph_labels[slic], segm_soft
-    torch = eng.torch
     early = {}
 
     def soft_sink(d_seg, d_proba):
-        # segm_soft = proba[slic] needs only the class probabilities: its gather and its (large) download run on a side stream
-        # while the main stream builds and cuts the graph
-        side = eng.side_stream()
-        side.wait_stream(torch.cuda.current_stream())
-        with torch.cuda.stream(side):
-            _, d_soft = eng.gather(d_seg, None, d_proba)
-            host = eng.pinned_empty(d_soft.shape, d_soft.dtype)
-            host.copy_(d_soft, non_blocking=True)
-            event = torch.cuda.Event()
-            event.record(side)
-        early['host'], early['event'] = host, event
+        early['host'], early['event'] = _soft_on_side_stream(eng, d_seg, d_proba)
 
     while True:
         early.clear()
         d_segm, d_soft, check = _run_resident(eng, image, model, dict_features, sp_size, sp_regul, gc_regul, gc_edge_type,
-                                              soft_sink=soft_sink if EARLY_SOFT_DOWNLOAD else None)
-        if check is None or not early:   # no graph cut / overlap switched off: both gathers were done at the end of the main stream
-            if check is not None:
-                segm, soft, n_edges = _download_results(eng, (d_segm, d_soft, check[0]))
-                if int(n_edges[0]) <= check[1]:
-                    break
-                EDGE_CAP_PER_NODE[0] *= 4
-                continue
+                                              soft_sink=soft_sink if EARLY_SOFT_DOWNLOAD else None, edge_cap=edge_cap)
+        if check is None:       # no graph cut: both gathers were done at the end of the main stream
             segm, soft = _download_results(eng, (d_segm, d_soft))
             break
-        segm, n_edges = _download_results(eng, (d_segm, check[0]))
-        early['event'].synchronize()
-        soft = early['host'].numpy()
-        # the next call reuses the buffers the side stream has just read: nothing of this call is left in flight
+        if early:
+            segm, n_edges = _download_results(eng, (d_segm, check[0]))
+            early['event'].synchronize()
+            soft = early['host'].numpy()
+            # the next call reuses the buffers the side stream has just read: nothing of this call is left in flight
+        else:                   # overlap switched off: segm_soft was gathered at the end of the main stream
+            segm, soft, n_edges = _download_results(eng, (d_segm, d_soft, check[0]))
         if int(n_edges[0]) <= check[1]:
             break
-        EDGE_CAP_PER_NODE[0] *= 4  # the device edge table overflowed (> 8 edges per superpixel on average): redo larger
+        edge_cap = grown_edge_capacity(check[1])     # the device edge table overflowed: redo larger
     if classes is not None:
         segm = np.asarray(classes)[segm]
     return segm, soft
@@ -306,6 +299,33 @@ def _batch_engines(nb_streams):
     while len(pool) < nb_streams:
         pool.append((Engine(dev), torch.cuda.Stream(device=dev)))
     return pool[:nb_streams]
+
+
+def _run_batch(list_images, nb_streams, max_in_flight, launch, finish):
+    """consecutive images alternate over ``nb_streams`` engines with a CUDA stream each, at most ``max_in_flight`` of them
+    unfinished.  ``launch(eng, image)`` queues one image's work and downloads on the current stream and returns (pinned host
+    tensors, their event, extra); ``finish(index, host arrays, extra)`` runs once the event has fired and gives the image's result.
+    Returns the results in input order."""
+    engines = _batch_engines(nb_streams)
+    torch = engines[0][0].torch
+    results, pending = [None] * len(list_images), []
+
+    def _finish(item):
+        idx, hosts, event, extra = item
+        event.synchronize()
+        results[idx] = finish(idx, [h.numpy() for h in hosts], extra)
+
+    caller_stream = torch.cuda.current_stream()
+    for i, image in enumerate(list_images):
+        eng, stream = engines[i % nb_streams]
+        stream.wait_stream(caller_stream)
+        with torch.cuda.stream(stream):
+            pending.append((i, ) + launch(eng, np.asarray(image)))
+        while len(pending) > max_in_flight:
+            _finish(pending.pop(0))
+    while pending:
+        _finish(pending.pop(0))
+    return results
 
 
 def segment_images_batch(list_images, nb_classes=None, dict_features=FTS_SET_SIMPLE, sp_size=30, sp_regul=0.2, use_scaler=True,
@@ -330,42 +350,22 @@ def segment_images_batch(list_images, nb_classes=None, dict_features=FTS_SET_SIM
                 for im in list_images]
     model = ('fit', nb_classes, use_scaler, 99) if model_pipeline is None else model_pipeline.predict_proba
     classes = getattr(model_pipeline, 'classes_', None)
-    engines = _batch_engines(nb_streams)
-    torch = engines[0][0].torch
-    results = [None] * len(list_images)
-    pending = []   # (index, pinned tensors, event, check)
 
-    def _finish(item):
-        idx, hosts, event, check = item
-        event.synchronize()
-        segm, soft = hosts[0].numpy(), hosts[1].numpy()
-        if check is not None and int(hosts[2].numpy()[0]) > check[1]:
-            EDGE_CAP_PER_NODE[0] *= 4  # edge table overflow (not seen in practice): redo this image through the single-image path
-            segm, soft = _segment(list_images[idx], model, dict_features, sp_size, sp_regul, gc_regul, gc_edge_type, None, classes=classes)
-        elif classes is not None:
+    def launch(eng, image):
+        d_segm, d_soft, check = _run_resident(eng, image, model, dict_features, sp_size, sp_regul, gc_regul, gc_edge_type)
+        return eng.download((d_segm, d_soft) + ((check[0], ) if check is not None else ())) + (check, )
+
+    def finish(idx, hosts, check):
+        segm, soft = hosts[0], hosts[1]
+        if check is not None and int(hosts[2][0]) > check[1]:
+            # edge table overflow (not seen in practice): redo this image through the single-image path with a larger table
+            return _segment(list_images[idx], model, dict_features, sp_size, sp_regul, gc_regul, gc_edge_type, None, classes=classes,
+                            edge_cap=grown_edge_capacity(check[1]))
+        if classes is not None:
             segm = np.asarray(classes)[segm]
-        results[idx] = (segm, soft)
+        return segm, soft
 
-    caller_stream = torch.cuda.current_stream()
-    for i, image in enumerate(list_images):
-        eng, stream = engines[i % nb_streams]
-        stream.wait_stream(caller_stream)
-        with torch.cuda.stream(stream):
-            d_segm, d_soft, check = _run_resident(eng, np.asarray(image), model, dict_features, sp_size, sp_regul, gc_regul, gc_edge_type)
-            tensors = (d_segm, d_soft) + ((check[0], ) if check is not None else ())
-            hosts = []
-            for t in tensors:
-                h = eng.pinned_empty(t.shape, t.dtype)
-                h.copy_(t, non_blocking=True)
-                hosts.append(h)
-            event = torch.cuda.Event()
-            event.record(stream)
-        pending.append((i, hosts, event, check))
-        while len(pending) > max_in_flight:
-            _finish(pending.pop(0))
-    while pending:
-        _finish(pending.pop(0))
-    return results
+    return _run_batch(list_images, nb_streams, max_in_flight, launch, finish)
 
 
 def compute_features_batch(list_images, dict_features, sp_size=30, sp_regul=0.2, nb_streams=3, max_in_flight=6):
@@ -377,34 +377,17 @@ def compute_features_batch(list_images, dict_features, sp_size=30, sp_regul=0.2,
     """
     if not flags_are_native(dict_features) or any(np.ndim(im) != 3 for im in list_images):
         return [compute_color2d_superpixels_features(im, dict_features, sp_size=sp_size, sp_regul=sp_regul)[1] for im in list_images]
-    engines = _batch_engines(nb_streams)
-    torch = engines[0][0].torch
-    results, pending = [None] * len(list_images), []
 
-    def _finish(item):
-        idx, h_feat, h_n, event = item
-        event.synchronize()
-        features = h_feat.numpy()[:int(h_n.numpy()[0])].copy()
+    def launch(eng, image):
+        res = _device_slic_features(eng, image, dict_features, sp_size, sp_regul)
+        return eng.download((res.d_feat, res.d_n_labels)) + (None, )
+
+    def finish(idx, hosts, _):
+        features = hosts[0][:int(hosts[1][0])].copy()
         features[np.isnan(features)] = 0
-        results[idx] = features
+        return features
 
-    caller_stream = torch.cuda.current_stream()
-    for i, image in enumerate(list_images):
-        eng, stream = engines[i % nb_streams]
-        stream.wait_stream(caller_stream)
-        with torch.cuda.stream(stream):
-            res = _device_slic_features(eng, np.asarray(image), dict_features, sp_size, sp_regul)
-            h_feat, h_n = eng.pinned_empty(res.d_feat.shape, res.d_feat.dtype), eng.pinned_empty((1, ), torch.int32)
-            h_feat.copy_(res.d_feat, non_blocking=True)
-            h_n.copy_(res.d_n_labels, non_blocking=True)
-            event = torch.cuda.Event()
-            event.record(stream)
-        pending.append((i, h_feat, h_n, event))
-        while len(pending) > max_in_flight:
-            _finish(pending.pop(0))
-    while pending:
-        _finish(pending.pop(0))
-    return results
+    return _run_batch(list_images, nb_streams, max_in_flight, launch, finish)
 
 
 def wrapper_compute_color2d_slic_features_labels(img_annot, sp_size, sp_regul, dict_features, label_purity):

@@ -13,7 +13,7 @@ import logging
 
 import numpy as np
 
-from .engine import get_engine
+from .engine import get_engine, grown_edge_capacity
 
 #: spacing among neighboring pixels in axes X, Y, Z  (reference superpixels.py:19)
 IMAGE_SPACING = (1, 1, 1)
@@ -127,14 +127,14 @@ def get_segment_diffs_3d_conn6(grid):
 
 
 def device_adjacency(eng, d_seg, nb):
-    """(edges [E,2] int32 host array) of a device label map with labels in [0, nb); grows the table on overflow"""
+    """(device edges [cap, 2] int32, E) of a device label map or volume with labels in [0, nb); grows the table on overflow"""
     cap = None
     while True:
         edges, n_edges, cap = eng.adjacency(d_seg, nb, cap)
         E = int(eng.to_host(n_edges)[0])
         if E <= cap:
             return edges, E
-        cap *= 4
+        cap = grown_edge_capacity(cap)
 
 
 def make_graph_segm_connect_grid2d_conn4(grid):

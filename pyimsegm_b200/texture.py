@@ -6,13 +6,11 @@ Host side: the filter bank is built with numpy/scipy exactly like the reference 
 ``isb_lm_texture`` (correlation form, oriented batteries first, tf32 hi/lo split, operand layout).  The contraction, the battery max,
 the log-norm scaling and the per-superpixel statistics run in CUDA (``csrc/lm_texture.cu``).
 """
-import ctypes as C
 import itertools
 
 import numpy as np
 
-from . import _lib
-from .engine import FLAG_BITS, get_engine
+from .engine import dtype_code, flag_bits, get_engine
 
 #: sigma of the background that is subtracted before filtering (descriptors.py:1078)
 BACKGROUND_SIGMA = 150
@@ -131,25 +129,28 @@ def background_kernel(sigma=BACKGROUND_SIGMA, truncate=4.0):
     return np.ascontiguousarray(w), radius, np.ascontiguousarray(mix)
 
 
+def lm_setup(eng, bank_type, flags):
+    """what every launch of the Leung-Malik kernels takes besides the image: (names, d_w, NP, orient, n_batt, w_bg, radius, mix,
+    bits, ncol) -- the uploaded bank (:func:`_device_bank`), the background kernel (:func:`background_kernel`; the caller puts its
+    taps ``w_bg`` on the device with ``eng.const_device(w_bg, 'lm_bg_w')``), the statistics' bit mask and the number of feature
+    columns"""
+    names, d_w, NP, orient, n_batt = _device_bank(bank_type)
+    w_bg, radius, mix = background_kernel()
+    bits, n = flag_bits(flags)
+    return names, d_w, NP, orient, n_batt, w_bg, radius, mix, bits, n_batt * 3 * n
+
+
 def device_lm_features(eng, d_img, d_seg, nb, flags, bank_type='normal', feat=None, col0=0):
     """run isb_lm_texture on device buffers; returns (feat tensor [nb, ld], names, n_cols)"""
-    torch, lib = eng.torch, eng.lib
-    names, d_w, NP, orient, n_batt = _device_bank(bank_type)
-    bits = 0
-    for f in flags:
-        bits |= FLAG_BITS[f]
-    ncol = n_batt * 3 * bin(bits).count('1')
+    names, d_w, NP, orient, n_batt, w_bg, radius, mix, bits, ncol = lm_setup(eng, bank_type, flags)
+    nb = int(nb)
     if feat is None:
-        feat = eng.buf('feat_lm', (nb, ncol), torch.float64)
+        feat = eng.buf('feat_lm', (nb, ncol), eng.torch.float64)
     H, W = int(d_seg.shape[0]), int(d_seg.shape[1])
-    w_bg, radius, mix = background_kernel()
     d_wbg = eng.const_device(w_bg, 'lm_bg_w')
-    wsb = lib.isb_lm_workspace_bytes(H, W, int(nb), n_batt)
-    ws = eng.buf('ws_lm', (wsb,), torch.uint8)
-    code = _lib.DTYPE_CODES[str(d_img.dtype).replace('torch.', '')]
-    _lib.check(lib.isb_lm_texture(_lib.ptr(d_img), code, _lib.ptr(d_seg), H, W, int(nb), _lib.ptr(d_wbg), radius,
-                                  mix.ctypes.data_as(C.POINTER(C.c_double)), _lib.ptr(d_w), NP, orient, n_batt, bits,
-                                  _lib.ptr(feat), int(feat.shape[1]), int(col0), _lib.ptr(ws), C.c_size_t(wsb), _lib.stream_ptr()))
+    ws, wsb = eng.workspace('ws_lm', 'lm_workspace_bytes', H, W, nb, n_batt)
+    eng.call('lm_texture', d_img, dtype_code(d_img.dtype), d_seg, H, W, nb, d_wbg, radius, mix, d_w, NP, orient, n_batt, bits, feat,
+             int(feat.shape[1]), int(col0), ws, wsb)
     return feat, names, ncol
 
 

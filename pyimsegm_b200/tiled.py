@@ -20,13 +20,12 @@ back to the whole image on its own GPU).
 Several bands may live on one GPU (``bands_per_rank``); the merge between them is the same integer sum done by
 ``isb_combine`` -- that is also how the single-GPU tests exercise every code path of the exchange.
 """
-import ctypes as C
 import logging
 
 import numpy as np
 
 from . import _lib
-from .engine import FLAG_BITS, gaussian_half_kernel, get_engine, slic_seed_grid
+from .engine import dtype_code, flag_bits, get_engine, grown_edge_capacity
 
 OP_SUM_I64, OP_MAX_I64, OP_MIN_F64, OP_MAX_F64, OP_SUM_F64 = 0, 1, 2, 3, 4
 
@@ -101,10 +100,6 @@ class TiledSuperpixels(object):
     fell_back = False
 
 
-def _combine(lib, dst_ptr, src_ptr, n, op):
-    _lib.check(lib.isb_combine(C.c_void_p(dst_ptr), C.c_void_p(src_ptr), C.c_longlong(int(n)), int(op), _lib.stream_ptr()))
-
-
 def slic_tiled(image, n_segments, compactness, sigma=1.0, max_iter=10, slic_zero=False, rescale=True, comm=None,
                bands_per_rank=1, eng=None, min_size_factor=0.5, max_size_factor=3, enforce_connectivity=True, defer_check=False,
                force_whole=False, raw_margin=0):
@@ -120,22 +115,15 @@ def slic_tiled(image, n_segments, compactness, sigma=1.0, max_iter=10, slic_zero
         the rows ``bands[local[i]].up_lo:up_hi``) -- the Leung-Malik descriptor needs its background radius + 16
     """
     eng = eng or get_engine()
-    torch, lib = eng.torch, eng.lib
+    torch = eng.torch
     comm = comm or default_comm()
     image = np.asarray(image)
     if image.ndim == 2:
         image = image[:, :, None]
     H, W, Cn = int(image.shape[0]), int(image.shape[1]), int(image.shape[2])
-    code = _lib.DTYPE_CODES[str(image.dtype)]
-    itemsize = image.dtype.itemsize
-    st = _lib.stream_ptr()
-    if sigma > 0:
-        w_half, radius = gaussian_half_kernel(sigma)
-    else:
-        w_half, radius = np.ones(1), 0
-    seeds, ty, tx = slic_seed_grid(H, W, n_segments)
+    code = dtype_code(image.dtype)
+    w_half, radius, seeds, ty, tx, step = eng.slic_setup(H, W, n_segments, sigma)
     n_seeds = len(seeds)
-    step = float(max(1, ty, tx))
     halo = 2 * ty + 1
     n_bands = comm.world * int(bands_per_rank)
     bands = plan_bands(H, n_bands, halo, radius, int(raw_margin))
@@ -147,7 +135,7 @@ def slic_tiled(image, n_segments, compactness, sigma=1.0, max_iter=10, slic_zero
     d_seeds = eng.to_device(seeds, 'seeds')
     mm = eng.buf('tb_minmax', (4,), torch.float64)
     mm_b = eng.buf('tb_minmax_b', (4,), torch.float64)
-    wsb = lib.isb_slic_kmeans_workspace_bytes(H, W, n_seeds, ty, tx)
+    wsb = eng.query('slic_kmeans_workspace_bytes', H, W, n_seeds, ty, tx)
 
     # 1) upload the raw rows, extrema of the owned rows
     res.d_raw = []
@@ -156,12 +144,11 @@ def slic_tiled(image, n_segments, compactness, sigma=1.0, max_iter=10, slic_zero
         raw = eng.to_device(image[bd.up_lo:bd.up_hi], 'tb%d_raw' % i)
         res.d_raw.append(raw)
         if rescale:
-            own_ptr = raw.data_ptr() + (bd.own_lo - bd.up_lo) * W * Cn * itemsize
-            tgt = mm if i == 0 else mm_b
-            _lib.check(lib.isb_image_minmax(C.c_void_p(own_ptr), code, C.c_longlong((bd.own_hi - bd.own_lo) * W * Cn), _lib.ptr(tgt), st))
+            eng.call('image_minmax', raw[bd.own_lo - bd.up_lo:bd.own_hi - bd.up_lo], code, (bd.own_hi - bd.own_lo) * W * Cn,
+                     mm if i == 0 else mm_b)
             if i > 0:
-                _combine(lib, mm.data_ptr(), mm_b.data_ptr(), 1, OP_MIN_F64)
-                _combine(lib, mm.data_ptr() + 8, mm_b.data_ptr() + 8, 1, OP_MAX_F64)
+                eng.call('combine', mm, mm_b, 1, OP_MIN_F64)
+                eng.call('combine', mm[1:2], mm_b[1:2], 1, OP_MAX_F64)
     if rescale:
         comm.all_reduce(mm[0:1], 'min')
         comm.all_reduce(mm[1:2], 'max')
@@ -176,37 +163,36 @@ def slic_tiled(image, n_segments, compactness, sigma=1.0, max_iter=10, slic_zero
         bd = bands[b]
         hraw = bd.raw_hi - bd.raw_lo
         lab = eng.buf('tb%d_lab' % i, (3, hraw, W), torch.float64)
-        raw_ptr = C.c_void_p(res.d_raw[i].data_ptr() + (bd.raw_lo - bd.up_lo) * W * Cn * itemsize)
-        _lib.check(lib.isb_slic_prepare(raw_ptr, code, hraw, W, Cn, w_half.ctypes.data_as(C.POINTER(C.c_double)), radius,
-                                        C.c_double(1.0 / compactness), 2 if rescale else 0, _lib.ptr(lab), _lib.ptr(mm), st))
+        eng.call('slic_prepare', res.d_raw[i][bd.raw_lo - bd.up_lo:bd.raw_hi - bd.up_lo], code, hraw, W, Cn, w_half, radius,
+                 1.0 / compactness, 2 if rescale else 0, lab, mm)
         slab_rows = bd.km_hi - bd.km_lo
         labels = eng.buf('tb%d_labels' % i, (slab_rows, W), torch.int32)
         ws = eng.buf('tb%d_ws' % i, (wsb,), torch.uint8)
         d = _lib.SlicBand(slab_rows=slab_rows, width=W, image_rows=H, y_off=bd.km_lo, own_lo=bd.own_lo, own_hi=bd.own_hi, halo=halo,
                           n_seeds=n_seeds, step_y=ty, step_x=tx, slic_zero=int(bool(slic_zero)), step=step,
-                          lab_slab=lab.data_ptr() + (bd.km_lo - bd.raw_lo) * W * 8, plane_stride=hraw * W,
+                          lab_slab=lab[:, bd.km_lo - bd.raw_lo:].data_ptr(), plane_stride=hraw * W,
                           seeds_yx=d_seeds.data_ptr(), labels_slab=labels.data_ptr(), ws=ws.data_ptr(), ws_bytes=wsb)
         descs.append(d)
         keep.append((lab, labels, ws))
-        _lib.check(lib.isb_slic_band_begin(C.byref(d), st))
+        eng.call('slic_band_begin', d)
 
     # 3) the sweeps: assign, sum the owned clusters, merge, take the merged centroids
     for _ in range(0 if force_whole else int(max_iter)):
         for i, d in enumerate(descs):
-            _lib.check(lib.isb_slic_band_assign(C.byref(d), st))
-            _lib.check(lib.isb_slic_band_update(C.byref(d), _lib.ptr(xchg[i]), st))
+            eng.call('slic_band_assign', d)
+            eng.call('slic_band_update', d, xchg[i])
             if i > 0:
-                _combine(lib, xchg[0].data_ptr(), xchg[i].data_ptr(), 6 * n_seeds + 1, OP_SUM_I64)
+                eng.call('combine', xchg[0], xchg[i], 6 * n_seeds + 1, OP_SUM_I64)
         comm.all_reduce(xchg[0], 'sum')
-        _combine(lib, err.data_ptr(), xchg[0].data_ptr() + 8 * 6 * n_seeds, 1, OP_SUM_I64)
+        eng.call('combine', err, xchg[0][6 * n_seeds:], 1, OP_SUM_I64)
         for i, d in enumerate(descs):
-            _lib.check(lib.isb_slic_band_import(C.byref(d), _lib.ptr(xchg[0]), _lib.ptr(mdc[i]), st))
+            eng.call('slic_band_import', d, xchg[0], mdc[i])
             if slic_zero and i > 0:
-                _combine(lib, mdc[0].data_ptr(), mdc[i].data_ptr(), n_seeds, OP_MAX_I64)
+                eng.call('combine', mdc[0], mdc[i], n_seeds, OP_MAX_I64)
         if slic_zero:
             comm.all_reduce(mdc[0], 'max')
         for d in descs:
-            _lib.check(lib.isb_slic_band_finalize(C.byref(d), _lib.ptr(mdc[0]), st))
+            eng.call('slic_band_finalize', d, mdc[0])
 
     # 4) the whole k-means label map on every GPU
     full = eng.buf('tb_full', (H, W), torch.int32)
@@ -230,15 +216,7 @@ def slic_tiled(image, n_segments, compactness, sigma=1.0, max_iter=10, slic_zero
     if not enforce_connectivity:
         res.d_seg = full
         return res
-    segment_size = 1 * H * W / n_segments
-    min_size, max_size = int(min_size_factor * segment_size), int(max_size_factor * segment_size)
-    cwsb = lib.isb_connectivity_workspace_bytes(H, W)
-    cws = eng.buf('ws_conn', (cwsb,), torch.uint8)
-    out = eng.buf('labels', (H, W), torch.int32)
-    n_labels = eng.buf('n_labels', (1,), torch.int32)
-    _lib.check(lib.isb_enforce_connectivity(_lib.ptr(full), H, W, min_size, max_size, _lib.ptr(out), _lib.ptr(n_labels), _lib.ptr(cws),
-                                            C.c_size_t(cwsb), st))
-    res.d_seg, res.d_n_labels = out, n_labels
+    res.d_seg, res.d_n_labels = eng.connectivity(full, n_segments, min_size_factor, max_size_factor)
     res.nb_bound = eng.slic_label_bound(H, W, n_segments, min_size_factor)
     return res
 
@@ -247,18 +225,14 @@ def color_stats_tiled(res, image_dtype, channels, flags, comm=None, eng=None, fe
     """colour statistics + centroids of the banded image over ``res.d_seg``: every band accumulates its owned rows, the
     accumulators are summed over the GPUs, every GPU finishes the same [nb, 3*len(flags)] table"""
     eng = eng or get_engine()
-    torch, lib = eng.torch, eng.lib
+    torch = eng.torch
     comm = comm or default_comm()
-    H, W = res.shape
+    W = res.shape[1]
     if channels != 3:
         raise ValueError('the colour statistics need a 3-channel image')
-    code = _lib.DTYPE_CODES[str(np.dtype(image_dtype))]
-    itemsize = np.dtype(image_dtype).itemsize
+    code = dtype_code(image_dtype)
     nb = int(res.nb_bound)
-    st = _lib.stream_ptr()
-    bits = 0
-    for f in flags:
-        bits |= FLAG_BITS[f]
+    bits, n = flag_bits(flags)
     acc = eng.buf('tb_acc', (nb, 6), torch.float64)
     iacc = eng.buf('tb_iacc', (nb, 3), torch.int64)
     acc.zero_()
@@ -266,14 +240,11 @@ def color_stats_tiled(res, image_dtype, channels, flags, comm=None, eng=None, fe
 
     def rows(i, b):
         bd = res.bands[b]
-        img_ptr = res.d_raw[i].data_ptr() + (bd.own_lo - bd.up_lo) * W * 3 * itemsize
-        seg_ptr = res.d_seg.data_ptr() + bd.own_lo * W * 4
-        return bd, C.c_void_p(img_ptr), C.c_void_p(seg_ptr)
+        return bd, res.d_raw[i][bd.own_lo - bd.up_lo:bd.own_hi - bd.up_lo], res.d_seg[bd.own_lo:bd.own_hi]
 
     for i, b in enumerate(res.local):
-        bd, img_ptr, seg_ptr = rows(i, b)
-        _lib.check(lib.isb_segment_stats_accumulate(img_ptr, code, seg_ptr, bd.own_hi - bd.own_lo, W, bd.own_lo, nb, _lib.ptr(acc),
-                                                    _lib.ptr(iacc), st))
+        bd, img, seg = rows(i, b)
+        eng.call('segment_stats_accumulate', img, code, seg, bd.own_hi - bd.own_lo, W, bd.own_lo, nb, acc, iacc)
     comm.all_reduce(acc, 'sum')
     comm.all_reduce(iacc, 'sum')
     var = None
@@ -282,16 +253,13 @@ def color_stats_tiled(res, image_dtype, channels, flags, comm=None, eng=None, fe
         meanf = eng.buf('tb_meanf', (nb, 3), torch.float32)
         var.zero_()
         for i, b in enumerate(res.local):
-            bd, img_ptr, seg_ptr = rows(i, b)
-            _lib.check(lib.isb_segment_stats_deviation(img_ptr, code, seg_ptr, bd.own_hi - bd.own_lo, W, nb, _lib.ptr(acc), _lib.ptr(iacc),
-                                                       _lib.ptr(meanf), _lib.ptr(var), st))
+            bd, img, seg = rows(i, b)
+            eng.call('segment_stats_deviation', img, code, seg, bd.own_hi - bd.own_lo, W, nb, acc, iacc, meanf, var)
         comm.all_reduce(var, 'sum')
-    ncol = 3 * bin(bits).count('1')
     if feat is None:
-        feat = eng.buf('feat', (nb, max(ncol, 1)), torch.float64)
+        feat = eng.buf('feat', (nb, max(3 * n, 1)), torch.float64)
     centres = eng.buf('centres', (nb, 2), torch.float64)
-    _lib.check(lib.isb_segment_stats_finish(nb, bits, _lib.ptr(acc), _lib.ptr(var), _lib.ptr(iacc), _lib.ptr(feat), int(feat.shape[1]),
-                                            int(col0), _lib.ptr(centres), None, st))
+    eng.call('segment_stats_finish', nb, bits, acc, var, iacc, feat, int(feat.shape[1]), int(col0), centres, None)
     res.d_feat, res.d_centres = feat, centres
     return feat, centres
 
@@ -305,22 +273,16 @@ def texture_stats_tiled(res, image_dtype, flags, bank_type='normal', comm=None, 
     have been called with ``raw_margin=LM_ROW_MARGIN``) and accumulates the sums of the rows it owns; the accumulators -- the
     per-superpixel sums and the per-battery response norms of the WHOLE image -- are summed over the GPUs, every GPU finishes
     the same [nb, n_batteries * 3 * len(flags)] block of ``feat``"""
-    from .texture import _device_bank, background_kernel
+    from .texture import lm_setup
     eng = eng or get_engine()
-    torch, lib = eng.torch, eng.lib
+    torch = eng.torch
     comm = comm or default_comm()
     H, W = res.shape
-    code = _lib.DTYPE_CODES[str(np.dtype(image_dtype))]
-    itemsize = np.dtype(image_dtype).itemsize
+    code = dtype_code(image_dtype)
     nb = int(res.nb_bound)
-    st = _lib.stream_ptr()
-    bits = 0
-    for f in flags:
-        bits |= FLAG_BITS[f]
-    _, d_w, NP, orient, n_batt = _device_bank(bank_type)
-    w_bg, radius, mix = background_kernel()
+    _, d_w, NP, orient, n_batt, w_bg, radius, mix, bits, ncol = lm_setup(eng, bank_type, flags)
     d_wbg = eng.const_device(w_bg, 'lm_bg_w')
-    acc = eng.buf('tb_lm_acc', (int(lib.isb_lm_acc_doubles(nb, n_batt)),), torch.float64)
+    acc = eng.buf('tb_lm_acc', (int(eng.query('lm_acc_doubles', nb, n_batt)),), torch.float64)
     counts = eng.buf('tb_lm_counts', (nb,), torch.int32)
     acc.zero_()
     counts.zero_()
@@ -330,19 +292,14 @@ def texture_stats_tiled(res, image_dtype, flags, bank_type='normal', comm=None, 
         if lo < bd.up_lo or hi > bd.up_hi:
             raise ValueError('the band keeps the raw rows %d:%d, the texture descriptor needs %d:%d (slic_tiled raw_margin)'
                              % (bd.up_lo, bd.up_hi, lo, hi))
-        img_ptr = C.c_void_p(res.d_raw[i].data_ptr() + (lo - bd.up_lo) * W * 3 * itemsize)
-        seg_ptr = C.c_void_p(res.d_seg.data_ptr() + lo * W * 4)
-        wsb = lib.isb_lm_workspace_bytes(hi - lo, W, nb, n_batt)
-        ws = eng.buf('ws_lm', (wsb,), torch.uint8)
-        _lib.check(lib.isb_lm_texture_accumulate(img_ptr, code, seg_ptr, hi - lo, W, bd.own_lo - lo, bd.own_hi - lo, nb, _lib.ptr(d_wbg), radius,
-                                                 mix.ctypes.data_as(C.POINTER(C.c_double)), _lib.ptr(d_w), NP, orient, n_batt,
-                                                 _lib.ptr(acc), _lib.ptr(counts), _lib.ptr(ws), C.c_size_t(wsb), st))
+        ws, wsb = eng.workspace('ws_lm', 'lm_workspace_bytes', hi - lo, W, nb, n_batt)
+        eng.call('lm_texture_accumulate', res.d_raw[i][lo - bd.up_lo:hi - bd.up_lo], code, res.d_seg[lo:hi], hi - lo, W, bd.own_lo - lo,
+                 bd.own_hi - lo, nb, d_wbg, radius, mix, d_w, NP, orient, n_batt, acc, counts, ws, wsb)
     comm.all_reduce(acc, 'sum')
     comm.all_reduce(counts, 'sum')
-    ncol = n_batt * 3 * bin(bits).count('1')
     if feat is None:
         feat = eng.buf('feat_lm', (nb, ncol), torch.float64)
-    _lib.check(lib.isb_lm_texture_finish(nb, n_batt, bits, _lib.ptr(acc), _lib.ptr(counts), _lib.ptr(feat), int(feat.shape[1]), int(col0), st))
+    eng.call('lm_texture_finish', nb, n_batt, bits, acc, counts, feat, int(feat.shape[1]), int(col0))
     return feat
 
 
@@ -375,8 +332,7 @@ def pipe_color2d_slic_features_model_graphcut_tiled(image, nb_classes, dict_feat
     """
     from . import graph_cuts
     from .descriptors import flags_are_native, native_feature_layout
-    from .graph_cuts import compute_pairwise_cost
-    from .pipelines import EDGE_CAP_PER_NODE, _edge_mode
+    from .pipelines import _device_graphcut, _soft_on_side_stream
     from .superpixels import _as_rgb_like, _supported_dtype, slic_params
     if sp_regul <= 0.:
         raise ValueError('slic. regularisation must be positive')
@@ -387,17 +343,15 @@ def pipe_color2d_slic_features_model_graphcut_tiled(image, nb_classes, dict_feat
                                   % dict_features)
     margin = LM_ROW_MARGIN if any(k.startswith('tLM') for k, _, _, _ in layout) else 0
     eng = get_engine()
-    torch, lib = eng.torch, eng.lib
     comm = comm or default_comm()
     image = _supported_dtype(_as_rgb_like(np.asarray(image)))
     H, W = int(image.shape[0]), int(image.shape[1])
     n_seg, compact = slic_params((H, W), sp_size, sp_regul)
     if n_seg < 1:
         raise ValueError('superpixel size %r is larger than the image %r' % (sp_size, tuple(image.shape)))
-    st = _lib.stream_ptr()
     K = int(nb_classes)
     n_init = max(1, int(np.sqrt(max_iter)))
-    force_whole, redo_front = False, True
+    force_whole, redo_front, cap = False, True, None
     while True:
         if redo_front:
             res = slic_tiled(image, n_seg, compact, sigma=1.0, comm=comm, bands_per_rank=bands_per_rank, eng=eng, defer_check=True,
@@ -407,56 +361,28 @@ def pipe_color2d_slic_features_model_graphcut_tiled(image, nb_classes, dict_feat
             d_proba, _ = eng.gmm_fit_predict(res.d_feat, K, n_init, max_iter, use_scaler, graph_cuts.RANDOM_SEED, d_n=res.d_n_labels)
             redo_front = False
         lo, hi = res.bands[res.local[0]].own_lo, res.bands[res.local[-1]].own_hi
-        rows = hi - lo
-        seg_ptr = C.c_void_p(res.d_seg.data_ptr() + lo * W * 4)
-        # segm_soft = proba[slic] of the owned rows needs only the class probabilities: its gather and its (large) download run on
-        # a side stream while the main stream builds and cuts the graph
         h_soft = soft_done = None
         if want_soft:
-            side = eng.side_stream()
-            side.wait_stream(torch.cuda.current_stream())
-            with torch.cuda.stream(side):
-                d_soft = eng.buf('segm_soft', (rows, W, K), torch.float64)
-                _lib.check(lib.isb_gather(seg_ptr, C.c_longlong(rows * W), None, _lib.ptr(d_proba), K, None, _lib.ptr(d_soft),
-                                          _lib.stream_ptr()))
-                h_soft = eng.pinned_empty(d_soft.shape, d_soft.dtype)
-                h_soft.copy_(d_soft, non_blocking=True)
-                soft_done = torch.cuda.Event()
-                soft_done.record(side)
-        cap = max(64, EDGE_CAP_PER_NODE[0] * nb)
-        pairwise = compute_pairwise_cost(gc_regul, (nb, K))
-        d_edges, d_n_edges, cap = eng.adjacency(res.d_seg, nb, cap)
-        _, _, unary_i, edge_wi, smooth_i = eng.gc_energies(d_proba, d_edges, cap, d_n_edges, res.d_centres, _edge_mode(gc_edge_type), 1.0,
-                                                           pairwise, d_n_nodes=res.d_n_labels)
-        d_labels, _, _ = eng.alpha_expansion(nb, K, cap, d_n_edges, d_edges, edge_wi, unary_i, smooth_i, -1, d_n_nodes=res.d_n_labels)
-        # 5) LUT gather of the owned rows
-        if gather_segm:
-            d_full = eng.buf('segm', (H, W), torch.int32)
-            d_segm = d_full[lo:hi]
-        else:
-            d_segm = eng.buf('segm', (rows, W), torch.int32)
-        _lib.check(lib.isb_gather(seg_ptr, C.c_longlong(rows * W), _lib.ptr(d_labels), None, K, _lib.ptr(d_segm), None, st))
+            h_soft, soft_done = _soft_on_side_stream(eng, res.d_seg[lo:hi], d_proba)
+        # 5) graph cut, LUT gather of the owned rows
+        _, d_segm, _, d_n_edges, cap = _device_graphcut(eng, res, nb, d_proba, gc_regul, gc_edge_type, d_n_nodes=res.d_n_labels,
+                                                        want_soft=False, edge_cap=cap, rows=(lo, hi), whole_segm=gather_segm)
+        d_full = eng.buf('segm', (H, W), eng.torch.int32) if gather_segm else None
         if gather_segm and comm.world > 1:
             for r in range(comm.world):
                 blo = res.bands[r * bands_per_rank].own_lo
                 bhi = res.bands[(r + 1) * bands_per_rank - 1].own_hi
                 comm.broadcast(d_full[blo:bhi], r)
-        outs = [d_full if gather_segm else d_segm, d_n_edges, res.d_err]
-        host = []
-        for t in outs:
-            h = eng.pinned_empty(t.shape, t.dtype)
-            h.copy_(t, non_blocking=True)
-            host.append(h)
-        torch.cuda.current_stream().synchronize()
+        (h_segm, h_n_edges, h_err), done = eng.download([d_segm if d_full is None else d_full, d_n_edges, res.d_err])
+        done.synchronize()
         if soft_done is not None:
             soft_done.synchronize()
-        host.append(h_soft)
-        if int(host[2][0]) != 0 and not force_whole:
+        if int(h_err[0]) != 0 and not force_whole:
             # orphan pixels beyond the halo (see slic_tiled): same answer on every rank, so every rank takes this branch
             logging.warning('banded SLIC met orphan pixels beyond the halo, redoing the sweeps on the whole image on every GPU')
             force_whole = redo_front = True
             continue
-        if int(host[1][0]) <= cap:
+        if int(h_n_edges[0]) <= cap:
             break
-        EDGE_CAP_PER_NODE[0] *= 4
-    return host[0].numpy(), (host[3].numpy() if want_soft else None), (lo, hi)
+        cap = grown_edge_capacity(cap)
+    return h_segm.numpy(), (h_soft.numpy() if want_soft else None), (lo, hi)

@@ -157,7 +157,7 @@ def test_config3_shaped_pipeline_with_a_shared_model(oracle):
 
 
 def test_cuda_graph_replay_equals_eager_launches():
-    """pipelines._run_resident_graph: the device part of the path captured once and replayed per image (batch API and
+    """pipelines._graph_call: the device part of the path captured once and replayed per image (batch API and
     segment_resident) must give exactly what the eager launches give, for every image of the batch"""
     from pyimsegm_b200 import pipelines as pl
     imgs = [synth_regions(200, 264, seed=s)[0] for s in (31, 32, 33, 34, 35)]
