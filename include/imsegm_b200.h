@@ -269,6 +269,19 @@ int isb_gmm_fit_predict(const double* feat, int N, int D, int ld, const int32_t*
                         double reg_covar, int use_scaler, unsigned long long seed, const int32_t* init_labels, double* proba,
                         double* params_out, void* ws, size_t ws_bytes, isb_stream_t stream);
 
+/* predict_proba of a GIVEN fitted mixture (GaussianMixture / BayesianGaussianMixture, any covariance type, optionally behind a
+ * StandardScaler), packed on the host into one device vector of isb_gmm_model_len(D, K) doubles:
+ *     shift[D] | scale[D] | U[K,D,D] | b[K,D] | c[K]
+ *   U_k: upper-triangular precision Cholesky factor (row-major, zeros below the diagonal), b_k = means_k U_k,
+ *   c_k: every term of log N_k + log weight_k that does not depend on the sample.
+ * For each row n < min(N, *n_dev): x = (f - shift) / scale with NaN features taken as 0, q_k = |x U_k - b_k|^2,
+ * lw_k = -(D log 2pi + q_k) / 2 + c_k, proba[n, k] = exp(lw_k - logsumexp(lw)).  Rows at or beyond the count are not written.
+ * D <= 16 needs no workspace; 16 < D <= 232 runs the batched FP64 GEMM of the fit (K <= 8). */
+int isb_gmm_model_len(int D, int K);
+size_t isb_gmm_predict_workspace_bytes(int N, int D, int K);
+int isb_gmm_predict(const double* feat, int N, int D, int ld, const int32_t* n_dev, int K, const double* model, double* proba, void* ws,
+                    size_t ws_bytes, isb_stream_t stream);
+
 /* compute_texture_desc_lm_img2d_clr (imsegm/descriptors.py:1041-1106): sigma-150 background subtraction (reflect, all three
  * axes), Leung-Malik filter bank (33x33 kernels) as an implicit GEMM on the tensor cores (tcgen05.mma kind::tf32 with the 3xTF32
  * split, FP32 accumulators in tensor memory, operands staged by TMA), max over the orientations of a battery, clip at 1e6,

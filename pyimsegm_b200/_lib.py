@@ -72,7 +72,10 @@ SIGNATURES = {
     'isb_gmm_workspace_bytes': (_sz, [_i, _i, _i, _i]),
     'isb_gmm_params_len': (_i, [_i, _i]),
     'isb_gmm_fit_predict': (_i, [_vp, _i, _i, _i, _vp, _i, _i, _i, _d, _d, _i, C.c_ulonglong, _vp, _vp, _vp, _vp, _sz, _vp]),
-    'isb_lm_workspace_bytes': (_sz, [_i, _i, _i, _i]),
+    'isb_gmm_model_len': (_i, [_i, _i]),
+    'isb_gmm_predict_workspace_bytes': (_sz, [_i, _i, _i]),
+    'isb_gmm_predict': (_i, [_vp, _i, _i, _i, _vp, _i, _vp, _vp, _vp, _sz, _vp]),
+    'isb_lm_workspace_bytes':(_sz, [_i, _i, _i, _i]),
     'isb_lm_acc_doubles': (_sz, [_i, _i]),
     'isb_lm_texture_accumulate': (_i, [_vp, _i, _vp, _i, _i, _i, _i, _i, _vp, _i, C.POINTER(_d), _vp, _i, _i, _i, _vp, _vp, _vp, _sz, _vp]),
     'isb_lm_texture_finish': (_i, [_i, _i, _i, _vp, _vp, _vp, _i, _i, _vp]),

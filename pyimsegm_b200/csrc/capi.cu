@@ -15,7 +15,7 @@ void isb_set_error(const char* fmt, ...)
 }
 
 extern "C" const char* isb_last_error(void) { return g_err; }
-extern "C" int isb_abi_version(void) { return 5; }  // 5: banded Leung-Malik statistics (accumulate / finish), tcgen05 issue-rate probe; 4: tcgen05 operand layout (w_tc), UMMA self-test, graph replay accounting, segment median
+extern "C" int isb_abi_version(void) { return 6; }  // 6: predict_proba of a given mixture model (isb_gmm_predict); 5: banded Leung-Malik statistics (accumulate / finish), tcgen05 issue-rate probe; 4: tcgen05 operand layout (w_tc), UMMA self-test, graph replay accounting, segment median
 extern "C" long long isb_launch_count(void) { return g_isb_launches; }
 extern "C" int isb_note_graph_replay(long long n_kernels) { g_isb_launches += n_kernels; return ISB_OK; }
 

@@ -1033,8 +1033,14 @@ __global__ void k_big_best(int D, int K, int n_init, GmmWs w)
     *w.flag = best;
 }
 
-// predict_proba of the best restart from Y = X U (in w.big, slots 0..K-1), and the exported parameters
-__global__ void __launch_bounds__(256) k_big_proba(int N_in, const int* n_dev, int D, int K, int best, GmmWs w, double* proba, double* params_out)
+// what k_big_proba copies out after a fit: scaler, the winning restart's parameters and its index (out == nullptr: nothing)
+struct ParamExport { const double* scale; const double* par; int best; double* out; };
+
+// predict_proba from Y = X U ([K, N_in, D]: component k's rows at Y + k N_in D), b_k = mu_k U_k ([K, D]) and the per-component
+// constants c ([K]: log|prec_chol_k| + log w_k, or whatever else does not depend on the sample); warp per sample
+__global__ void __launch_bounds__(256) k_big_proba(int N_in, const int* n_dev, int D, int K, const double* __restrict__ Y,
+                                                   const double* __restrict__ bvec, const double* __restrict__ cvec, double* proba,
+                                                   ParamExport ex)
 {
     const int N = n_dev ? min(*n_dev, N_in) : N_in;
     const int lane = threadIdx.x & 31, wl = threadIdx.x >> 5;
@@ -1043,13 +1049,13 @@ __global__ void __launch_bounds__(256) k_big_proba(int N_in, const int* n_dev, i
         double lw[KMAX];
         double mx = -DBL_MAX;
         for (int k = 0; k < K; ++k) {
-            const double* y = w.big + ((size_t)k * N_in + n) * D;
-            const double* b = w.bvec + ((size_t)best * K + k) * D;
+            const double* y = Y + ((size_t)k * N_in + n) * D;
+            const double* b = bvec + (size_t)k * D;
             double q = 0;
             for (int j = lane; j < D; j += 32) { const double t = y[j] - b[j]; q = fma(t, t, q); }
 #pragma unroll
             for (int o = 16; o > 0; o >>= 1) q += __shfl_xor_sync(0xffffffffu, q, o);
-            lw[k] = -0.5 * (D * 1.8378770664093453 + q) + w.ldw[best * K + k];
+            lw[k] = -0.5 * (D * 1.8378770664093453 + q) + cvec[k];
             mx = fmax(mx, lw[k]);
         }
         double s = 0;
@@ -1058,12 +1064,11 @@ __global__ void __launch_bounds__(256) k_big_proba(int N_in, const int* n_dev, i
         if (lane == 0)
             for (int k = 0; k < K; ++k) proba[(size_t)n * K + k] = exp(lw[k] - lse);
     }
-    if (blockIdx.x == 0 && params_out) {
+    if (blockIdx.x == 0 && ex.out) {
         const int ps = pstride(K, D);
-        const double* par = w.par + (size_t)best * ps;
-        for (int i = threadIdx.x; i < 2 * D; i += blockDim.x) params_out[i] = w.scale[i];
-        for (int i = threadIdx.x; i < ps; i += blockDim.x) params_out[2 * D + i] = par[i];
-        if (threadIdx.x == 0) params_out[2 * D + ps] = (double)best;
+        for (int i = threadIdx.x; i < 2 * D; i += blockDim.x) ex.out[i] = ex.scale[i];
+        for (int i = threadIdx.x; i < ps; i += blockDim.x) ex.out[2 * D + i] = ex.par[i];
+        if (threadIdx.x == 0) ex.out[2 * D + ps] = (double)ex.best;
     }
 }
 
@@ -1168,6 +1173,98 @@ __global__ void __launch_bounds__(256) k_gmm_predict(int N_in, const int* n_dev,
     }
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// predict_proba of a GIVEN model (isb_gmm_predict): a fitted GaussianMixture / BayesianGaussianMixture of any covariance type,
+// optionally behind a StandardScaler, packed on the host into one vector
+//     shift[D] | scale[D] | U[K, D, D] (upper-triangular precision Cholesky factors, zeros below) | b[K, D] = mu_k U_k | c[K]
+// lw_k = -1/2 (D log 2 pi + |x U_k - b_k|^2) + c_k with x = (nan -> 0 (f) - shift) / scale;  proba = softmax(lw).
+// Rows at or beyond the (device) sample count are neither read nor written.
+// ---------------------------------------------------------------------------------------------------------------------
+
+__host__ __device__ inline int model_len(int D, int K) { return 2 * D + K * D * D + K * D + K; }
+
+// D <= DMAX: one thread per sample, the model in shared memory, the standardised row and the K log-densities in registers
+// (every loop runs to its compile-time bound under a guard, so nothing is indexed at run time)
+constexpr int PT = 128;
+__global__ void __launch_bounds__(PT) k_model_predict(const double* __restrict__ feat, int N_in, int D, int ld, const int* n_dev, int K,
+                                                     const double* __restrict__ model, double* proba)
+{
+    __shared__ double s_m[2 * DMAX + KMAX * DMAX * DMAX + KMAX * DMAX + KMAX];
+    const int len = model_len(D, K);
+    for (int i = threadIdx.x; i < len; i += PT) s_m[i] = model[i];
+    __syncthreads();
+    const int N = n_dev ? min(*n_dev, N_in) : N_in;
+    const double* shift = s_m;
+    const double* scale = s_m + D;
+    const double* U = s_m + 2 * D;
+    const double* b = U + K * D * D;
+    const double* c = b + K * D;
+    for (int n = blockIdx.x * PT + threadIdx.x; n < N; n += gridDim.x * PT) {
+        double x[DMAX];
+#pragma unroll
+        for (int i = 0; i < DMAX; ++i) {
+            double f = 0.0;
+            if (i < D) {
+                f = feat[(size_t)n * ld + i];
+                f = isnan(f) ? 0.0 : f;
+                f = (f - shift[i]) / scale[i];
+            }
+            x[i] = f;
+        }
+        double lw[KMAX];
+        double mx = -DBL_MAX;
+#pragma unroll
+        for (int k = 0; k < KMAX; ++k) {
+            lw[k] = -DBL_MAX;
+            if (k < K) {
+                const double* Uk = U + k * D * D;
+                double q = 0;
+#pragma unroll
+                for (int j = 0; j < DMAX; ++j) {
+                    if (j < D) {
+                        double y = 0;
+#pragma unroll
+                        for (int i = 0; i <= j; ++i) y = fma(x[i], Uk[i * D + j], y);
+                        y -= b[k * D + j];
+                        q = fma(y, y, q);
+                    }
+                }
+                lw[k] = -0.5 * (D * 1.8378770664093453 + q) + c[k];
+                mx = fmax(mx, lw[k]);
+            }
+        }
+        double s = 0;
+#pragma unroll
+        for (int k = 0; k < KMAX; ++k) if (k < K) s += exp(lw[k] - mx);
+        const double lse = mx + log(s);
+#pragma unroll
+        for (int k = 0; k < KMAX; ++k) if (k < K) proba[(size_t)n * K + k] = exp(lw[k] - lse);
+    }
+}
+
+// DMAX < D: the standardised, NaN-cleaned rows [N, D] for the GEMM (rows below the sample count only)
+__global__ void __launch_bounds__(256) k_model_standardise(const double* __restrict__ feat, int N_in, int D, int ld, const int* n_dev,
+                                                           const double* __restrict__ model, double* __restrict__ xs)
+{
+    const int N = n_dev ? min(*n_dev, N_in) : N_in;
+    const size_t total = (size_t)N * D;
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
+        const int n = (int)(i / D), d = (int)(i % D);
+        double f = feat[(size_t)n * ld + d];
+        f = isnan(f) ? 0.0 : f;
+        xs[i] = (f - model[d]) / model[D + d];
+    }
+}
+
+static size_t carve_predict(void* ws, size_t bytes, int N, int D, int K, double** xs, double** ys)
+{
+    if (D <= DMAX) return 0;
+    WsCarver c(ws, bytes);
+    *xs = c.take<double>((size_t)N * D);
+    *ys = c.take<double>((size_t)K * N * D);
+    return isb_align(c.off);
+}
+
 static size_t carve_gmm(GmmWs& w, void* ws, size_t bytes, int N, int D, int K, int n_init)
 {
     WsCarver c(ws, bytes);
@@ -1221,7 +1318,9 @@ extern "C" int isb_gmm_fit_predict(const double* feat, int N, int D, int ld, con
         ISB_LAUNCH_CHECK();
         if (int rc = fit_big(N, n_dev, D, K, n_init, max_iter, tol, reg_covar, seed, init_labels, w, st, &best)) return rc;
         if (best >= 0) {
-            k_big_proba<<<(N + 7) / 8, 256, 0, st>>>(N, n_dev, D, K, best, w, proba, params_out);
+            const ParamExport ex = { w.scale, w.par + (size_t)best * pstride(K, D), best, params_out };
+            k_big_proba<<<(N + 7) / 8, 256, 0, st>>>(N, n_dev, D, K, w.big, w.bvec + (size_t)best * K * D, w.ldw + (size_t)best * K, proba,
+                                                     ex);
             ISB_LAUNCH_CHECK();
             return ISB_OK;
         }
@@ -1245,6 +1344,50 @@ extern "C" int isb_gmm_fit_predict(const double* feat, int N, int D, int ld, con
     int blocks = (N + 255) / 256;
     if (blocks > 148) blocks = 148;
     k_gmm_predict<<<blocks, 256, 0, st>>>(N, n_dev, D, K, n_init, w, proba, params_out);
+    ISB_LAUNCH_CHECK();
+    return ISB_OK;
+}
+
+extern "C" int isb_gmm_model_len(int D, int K) { return model_len(D, K); }
+
+extern "C" size_t isb_gmm_predict_workspace_bytes(int N, int D, int K)
+{
+    double *xs, *ys;
+    return carve_predict(nullptr, 0, N, D, K, &xs, &ys);
+}
+
+extern "C" int isb_gmm_predict(const double* feat, int N, int D, int ld, const int32_t* n_dev, int K, const double* model, double* proba,
+                               void* ws, size_t ws_bytes, isb_stream_t stream)
+{
+    ISB_REQUIRE(feat && model && proba, "null pointer");
+    ISB_REQUIRE(N > 0 && D > 0 && ld >= D && K > 0, "bad sizes");
+    if (D > DBIG || K > KMAX) { isb_set_error("device GMM handles D <= %d and K <= %d (got D=%d K=%d)", DBIG, KMAX, D, K); return ISB_ERR_UNSUPPORTED; }
+    cudaStream_t st = (cudaStream_t)stream;
+    ProfScope prof(ISB_PROF_GMM, st);
+    if (D <= DMAX) {
+        int blocks = (N + PT - 1) / PT;
+        if (blocks > 4 * 148) blocks = 4 * 148;
+        k_model_predict<<<blocks, PT, 0, st>>>(feat, N, D, ld, n_dev, K, model, proba);
+        ISB_LAUNCH_CHECK();
+        return ISB_OK;
+    }
+    double *xs = nullptr, *ys = nullptr;
+    ISB_REQUIRE(ws, "null pointer");
+    const size_t need = carve_predict(ws, ws_bytes, N, D, K, &xs, &ys);
+    ISB_REQUIRE(need <= ws_bytes, "workspace too small");
+    int blocks = (int)(((size_t)N * D + 255) / 256);
+    if (blocks > 8 * 148) blocks = 8 * 148;
+    k_model_standardise<<<blocks, 256, 0, st>>>(feat, N, D, ld, n_dev, model, xs);
+    ISB_LAUNCH_CHECK();
+    // Y_k = X U_k for every component in one launch (U_k upper triangular: column tiles skip the rows below them)
+    const size_t sND = (size_t)N * D, sDD = (size_t)D * D;
+    const BatchStride bs = { 0, 0, 0, sDD, 0, sND, 0 };
+    k_dgemm_batched<false, false><<<dim3((D + TN - 1) / TN, (N + TM - 1) / TM, K), 256, 0, st>>>(
+        xs, D, model + 2 * D, D, ys, D, bs, N, D, D, n_dev, 1, nullptr, K, 0, 1, 1, FuseW());
+    ISB_LAUNCH_CHECK();
+    const double* bvec = model + 2 * D + (size_t)K * sDD;
+    const ParamExport none = { nullptr, nullptr, 0, nullptr };
+    k_big_proba<<<(N + 7) / 8, 256, 0, st>>>(N, n_dev, D, K, ys, bvec, bvec + (size_t)K * D, proba, none);
     ISB_LAUNCH_CHECK();
     return ISB_OK;
 }

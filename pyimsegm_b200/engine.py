@@ -410,6 +410,15 @@ class Engine(object):
                   int(seed), d_init, proba, params, ws, wsb)
         return proba, params
 
+    def gmm_predict(self, d_feat, d_model, K, d_n=None):
+        """class probabilities [N, K] (the cached 'proba' buffer) of the features [N, D] under a GIVEN model, the device vector
+        packed by :class:`graph_cuts.DeviceClassModel` (see isb_gmm_predict); ``d_n``: device row count, rows beyond it untouched"""
+        N, D, K = int(d_feat.shape[0]), int(d_feat.shape[1]), int(K)
+        proba = self.buf('proba', (N, K), self.torch.float64)
+        ws, wsb = self.workspace('ws_gmm_predict', 'gmm_predict_workspace_bytes', N, D, K)
+        self.call('gmm_predict', d_feat, N, D, int(d_feat.stride(0)), d_n, K, d_model, proba, ws, wsb)
+        return proba
+
     def gather(self, d_seg, lut_i=None, lut_p=None, out_i=None):
         """segm = lut_i[seg] (into ``out_i`` or the cached 'segm') and segm_soft = lut_p[seg] over a device label map [H, W]"""
         torch = self.torch

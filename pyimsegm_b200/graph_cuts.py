@@ -4,7 +4,8 @@ GraphCut on the superpixel graph, on the GPU.
 Mirror of the reference module ``imsegm/graph_cuts.py`` (same public names, arguments, error types).  The graph,
 the energies and the alpha-expansion itself run in CUDA behind ``include/imsegm_b200.h``
 (``isb_adjacency_edges`` / ``isb_gc_energies`` / ``isb_alpha_expansion``); the class model stays scikit-learn
-exactly as in the reference (``estim_class_model``, reference graph_cuts.py:73-163).
+exactly as in the reference (``estim_class_model``, reference graph_cuts.py:73-163), fitted on the device when it is the default GMM
+(``isb_gmm_fit_predict``); a fitted mixture wrapped in :class:`DeviceClassModel` is evaluated on the device (``isb_gmm_predict``).
 """
 import logging
 
@@ -157,6 +158,131 @@ def estim_class_model_device(features, nb_classes, use_scaler=True, max_iter=99,
     _, params = eng.gmm_fit_predict(d_feat, nb_classes, n_init, max_iter, use_scaler, RANDOM_SEED if seed is None else seed,
                                     init_labels=None if init_labels is None else np.atleast_2d(init_labels))
     return sklearn_pipeline_from_device(eng.to_host(params), features.shape[1], nb_classes, len(features), use_scaler, n_init, max_iter)
+
+
+def _mixture_and_scaler(model):
+    """(StandardScaler or None, fitted mixture) of a model :class:`DeviceClassModel` can evaluate; ValueError naming the step it
+    cannot take"""
+    from sklearn import mixture, pipeline, preprocessing
+    steps = list(model.steps) if isinstance(model, pipeline.Pipeline) else [('model', model)]
+    for i, (name, step) in enumerate(steps[:-1]):
+        if i > 0 or not isinstance(step, preprocessing.StandardScaler):
+            raise ValueError('DeviceClassModel takes a mixture model behind at most one StandardScaler, not step %r (%s)'
+                             % (name, type(step).__name__))
+    name, mm = steps[-1]
+    if not isinstance(mm, (mixture.GaussianMixture, mixture.BayesianGaussianMixture)):
+        raise ValueError('DeviceClassModel evaluates a GaussianMixture or BayesianGaussianMixture, not step %r (%s)'
+                         % (name, type(mm).__name__))
+    if not hasattr(mm, 'precisions_cholesky_'):
+        raise ValueError('DeviceClassModel needs a fitted model (step %r is not fitted)' % name)
+    return (steps[0][1] if len(steps) > 1 else None), mm
+
+
+def pack_class_model(model):
+    """ the device vector of ``isb_gmm_predict`` for a fitted mixture model (optionally behind a StandardScaler):
+    shift[D] | scale[D] | U[K, D, D] | b[K, D] | c[K], computed the way scikit-learn's ``_estimate_log_gaussian_prob``,
+    ``_estimate_log_prob`` and ``_estimate_log_weights`` compute them (every covariance type expanded to a full triangular U_k)
+
+    :return tuple(ndarray, int, int): the vector, D, K
+    """
+    from scipy.special import digamma
+    from sklearn import mixture
+    scaler, mm = _mixture_and_scaler(model)
+    means = np.asarray(mm.means_, dtype=np.float64)
+    K, D = means.shape
+    if D > DEVICE_GMM_MAX_FEATURES or K > DEVICE_GMM_MAX_CLASSES:
+        raise ValueError('DeviceClassModel handles up to %d features and %d classes (got D=%d, K=%d)'
+                         % (DEVICE_GMM_MAX_FEATURES, DEVICE_GMM_MAX_CLASSES, D, K))
+    shift, scale = np.zeros(D), np.ones(D)
+    if scaler is not None:
+        if getattr(scaler, 'n_features_in_', D) != D:
+            raise ValueError('the StandardScaler has %d features, the mixture %d' % (scaler.n_features_in_, D))
+        if scaler.with_mean:
+            shift = np.asarray(scaler.mean_, dtype=np.float64)
+        if scaler.with_std:
+            scale = np.asarray(scaler.scale_, dtype=np.float64)
+    pc = np.asarray(mm.precisions_cholesky_, dtype=np.float64)
+    diag = np.arange(D)
+    ct = mm.covariance_type
+    U = np.zeros((K, D, D))
+    if ct == 'full':
+        U[:] = pc
+        log_det = np.log(pc[:, diag, diag]).sum(axis=1)
+    elif ct == 'tied':
+        U[:] = pc[None]
+        log_det = np.full(K, np.log(np.diag(pc)).sum())
+    elif ct == 'diag':
+        U[:, diag, diag] = pc
+        log_det = np.log(pc).sum(axis=1)
+    elif ct == 'spherical':
+        U[:, diag, diag] = pc[:, None]
+        log_det = D * np.log(pc)
+    else:
+        raise ValueError('unknown covariance_type %r' % ct)
+    b = np.einsum('kd,kde->ke', means, U)
+    if isinstance(mm, mixture.BayesianGaussianMixture):
+        dof = np.broadcast_to(np.asarray(mm.degrees_of_freedom_, dtype=np.float64), (K,))
+        log_lambda = D * np.log(2.0) + np.sum(digamma(0.5 * (dof - np.arange(D)[:, None])), 0)
+        c = log_det - 0.5 * D * np.log(dof) + 0.5 * (log_lambda - D / np.asarray(mm.mean_precision_, dtype=np.float64))
+        if mm.weight_concentration_prior_type == 'dirichlet_process':
+            a, bb = (np.asarray(v, dtype=np.float64) for v in mm.weight_concentration_)
+            dsum = digamma(a + bb)
+            log_w = digamma(a) - dsum + np.hstack((0, np.cumsum(digamma(bb) - dsum)[:-1]))
+        else:
+            conc = np.asarray(mm.weight_concentration_, dtype=np.float64)
+            log_w = digamma(conc) - digamma(np.sum(conc))
+        c = c + log_w
+    else:
+        c = log_det + np.log(np.asarray(mm.weights_, dtype=np.float64))
+    vec = np.concatenate([shift, scale, U.ravel(), b.ravel(), c]).astype(np.float64)
+    return np.ascontiguousarray(vec), int(D), int(K)
+
+
+class DeviceClassModel(object):
+    """ a fitted class model whose ``predict_proba`` runs on the GPU (``isb_gmm_predict``): a GaussianMixture or
+    BayesianGaussianMixture of any covariance type, bare or as the last step of a Pipeline whose only other step is a
+    StandardScaler -- every model the reference's ``estim_class_model`` builds without PCA.  Packed once, at construction.
+
+    Passed to ``segment_color2d_slic_features_model_graphcut``, ``segment_images_batch(model_pipeline=...)``,
+    ``segment_resident`` or ``tiled.segment_color2d_slic_features_model_graphcut_tiled`` it keeps the whole path on the device
+    (no feature download, no host model, CUDA-graph replays); a plain scikit-learn model keeps the host round trip.
+
+    :param model: the fitted scikit-learn object, kept as ``.model``; ``classes_`` is passed through when it has one
+    """
+
+    def __init__(self, model):
+        import hashlib
+        import weakref
+        self.model = model
+        self.params, self.n_features, self.n_classes = pack_class_model(model)
+        self.digest = hashlib.blake2b(self.params.tobytes(), digest_size=16).hexdigest()
+        classes = getattr(model, 'classes_', None)
+        if classes is not None:
+            self.classes_ = classes
+        self._on_device = weakref.WeakKeyDictionary()
+
+    def device_params(self, eng):
+        """the packed vector on ``eng``'s device (``Engine.const_device``: one tensor per engine and content, never overwritten);
+        call it outside a CUDA-graph capture"""
+        d = self._on_device.get(eng)
+        if d is None:
+            d = self._on_device[eng] = eng.const_device(self.params, 'class_model')
+        return d
+
+    def predict_proba(self, features):
+        """ class probabilities [N, K] of host features [N, D] (NaN taken as 0), computed on the device """
+        X = np.ascontiguousarray(features, dtype=np.float64)
+        if X.ndim != 2 or X.shape[1] != self.n_features:
+            raise ValueError('features of shape %r, the model takes %d columns' % (X.shape, self.n_features))
+        if not len(X):
+            return np.zeros((0, self.n_classes))
+        eng = get_engine()
+        d_feat = eng.to_device(X, 'feat_in')
+        proba = eng.gmm_predict(d_feat, self.device_params(eng), self.n_classes)
+        return eng.to_host(proba).copy()
+
+    def __repr__(self):
+        return 'DeviceClassModel(%r)' % (self.model, )
 
 
 def estim_class_model(features, nb_classes, estim_model='GMM', pca_coef=None, use_scaler=True, max_iter=99):

@@ -11,7 +11,8 @@ and return values):
 
 The image goes to the device once; label map, features, class model, graph, energies and the cut never leave it and the
 host synchronises ONCE, when the results are downloaded.  (A user-supplied model, or one the device GMM does not cover, costs
-one round trip: features [N, D] down, probabilities [N, K] up.)
+one round trip: features [N, D] down, probabilities [N, K] up -- unless it is wrapped in ``graph_cuts.DeviceClassModel``, whose
+probabilities are computed on the device.)
 """
 import logging
 
@@ -19,7 +20,7 @@ import numpy as np
 
 from .descriptors import FEATURES_SET_COLOR, compute_selected_features_img2d, flags_are_native, native_feature_layout
 from .engine import edge_capacity, get_engine, grown_edge_capacity
-from .graph_cuts import (_edge_mode, compute_pairwise_cost, device_gmm_applicable, estim_class_model,
+from .graph_cuts import (DeviceClassModel, _edge_mode, compute_pairwise_cost, device_gmm_applicable, estim_class_model,
                          segment_graph_cut_general)
 from .superpixels import _as_rgb_like, _supported_dtype, slic_params
 
@@ -171,33 +172,55 @@ def _features_key(dict_features):
     return tuple(sorted((k, tuple(v)) for k, v in dict_features.items()))
 
 
+def _check_model_width(model, dict_features):
+    """ValueError when a DeviceClassModel was fitted on another number of features than ``dict_features`` gives"""
+    ncol = native_feature_layout(dict_features)[1]
+    if ncol != model.n_features:
+        raise ValueError('the class model takes %d features, %r gives %d' % (model.n_features, dict_features, ncol))
+
+
 def _run_resident(eng, image, model, dict_features, sp_size, sp_regul, gc_regul, gc_edge_type, soft_sink=None, edge_cap=None):
     """the whole hot path on the device.  ``model`` is either ('fit', nb_classes, use_scaler, max_iter) -> the default
-    GMM is fitted on the GPU and NOTHING syncs with the host until the results are ready; or a callable
+    GMM is fitted on the GPU and NOTHING syncs with the host until the results are ready; or a :class:`DeviceClassModel` -> its
+    probabilities are evaluated on the GPU (isb_gmm_predict), again without a synchronisation; or a callable
     proba_fn(features) -> one round trip (features down, probabilities up) as in the reference.
     ``soft_sink(d_seg, d_proba)``: the caller takes ``segm_soft = proba[slic]`` itself as soon as the probabilities exist
     (it does not depend on the graph cut) -- then ``d_soft`` is returned as None.
-    With a device-fitted model and colour features the two halves -- image -> class probabilities, probabilities -> cut and LUT
+    With a device model and colour features the two halves -- image -> class probabilities, probabilities -> cut and LUT
     gathers -- are CUDA-graph replays (:func:`_graph_call`); the image then has to sit in one of the engine's cached buffers.
+    (The large-D fit synchronises once per EM iteration, so a fitted model is only captured up to 16 features; the prediction
+    never synchronises and is captured at any width.)
     ``edge_cap``: capacity of the edge table (default :func:`engine.edge_capacity` of the superpixel count).
     Returns (d_segm, d_soft, check): ``check`` is None or (d_n_edges, edge_cap) still to be verified by the caller."""
     no_cut = (not isinstance(gc_regul, (list, np.ndarray))) and gc_regul <= 0
-    if isinstance(model, tuple):
-        _, nb_classes, use_scaler, max_iter = model
+    if isinstance(model, (tuple, DeviceClassModel)):
         from . import graph_cuts
-        n_init = max(1, int(np.sqrt(max_iter)))
         if not hasattr(image, 'is_cuda'):
             image = eng.to_device(_supported_dtype(_as_rgb_like(np.asarray(image))), 'image')
-        graphable = (USE_CUDA_GRAPHS and not no_cut and all(k == 'color' for k in dict_features) and flags_are_native(dict_features)
-                     and native_feature_layout(dict_features)[1] <= graph_cuts.DEVICE_GMM_SINGLE_KERNEL_MAX_FEATURES)
+        graphable = (USE_CUDA_GRAPHS and not no_cut and all(k == 'color' for k in dict_features) and flags_are_native(dict_features))
+        if isinstance(model, DeviceClassModel):
+            _check_model_width(model, dict_features)
+            nb_classes = model.n_classes
+            d_model = model.device_params(eng)      # before any capture: const_device refuses a new constant while capturing
+            model_key = ('predict', model.digest)
+
+            def class_proba(res):
+                return eng.gmm_predict(res.d_feat, d_model, nb_classes, d_n=res.d_n_labels)
+        else:
+            _, nb_classes, use_scaler, max_iter = model
+            n_init = max(1, int(np.sqrt(max_iter)))
+            graphable = graphable and native_feature_layout(dict_features)[1] <= graph_cuts.DEVICE_GMM_SINGLE_KERNEL_MAX_FEATURES
+            model_key = model
+
+            def class_proba(res):
+                return eng.gmm_fit_predict(res.d_feat, nb_classes, n_init, max_iter, use_scaler, graph_cuts.RANDOM_SEED,
+                                           d_n=res.d_n_labels)[0]
 
         def first_half():
             res = _device_slic_features(eng, image, dict_features, sp_size, sp_regul)
-            d_proba, _ = eng.gmm_fit_predict(res.d_feat, nb_classes, n_init, max_iter, use_scaler, graph_cuts.RANDOM_SEED,
-                                             d_n=res.d_n_labels)
-            return res, d_proba
+            return res, class_proba(res)
 
-        key1 = ('probabilities', id(eng), image.data_ptr(), tuple(image.shape), str(image.dtype), model, _features_key(dict_features),
+        key1 = ('probabilities', id(eng), image.data_ptr(), tuple(image.shape), str(image.dtype), model_key, _features_key(dict_features),
                 sp_size, sp_regul)
         res, d_proba = _graph_call(eng, key1, first_half) if graphable else first_half()
         if no_cut:
@@ -246,7 +269,10 @@ def _segment(image, model, dict_features, sp_size, sp_regul, gc_regul, gc_edge_t
     native = image.ndim == 3 and flags_are_native(dict_features) and gc_edge_type not in ('color', 'features')
     if not native or debug_visual is not None:
         # general path: every stage still runs on the device, but through the numpy-facing stage functions
-        proba_fn = model if callable(model) else (lambda f: estim_class_model(f, model[1], 'GMM', None, model[2], model[3]).predict_proba(f))
+        if isinstance(model, DeviceClassModel):
+            proba_fn = model.predict_proba
+        else:
+            proba_fn = model if callable(model) else (lambda f: estim_class_model(f, model[1], 'GMM', None, model[2], model[3]).predict_proba(f))
         slic, features = compute_color2d_superpixels_features(image, dict_features, sp_size=sp_size, sp_regul=sp_regul)
         if debug_visual is not None:
             img3 = image if image.ndim == 3 else np.stack([image] * 3, axis=-1)
@@ -348,7 +374,10 @@ def segment_images_batch(list_images, nb_classes=None, dict_features=FTS_SET_SIM
     if not native:
         return [segment_color2d_slic_features_model_graphcut(im, model_pipeline, dict_features, sp_size, sp_regul, gc_regul, gc_edge_type)
                 for im in list_images]
-    model = ('fit', nb_classes, use_scaler, 99) if model_pipeline is None else model_pipeline.predict_proba
+    if model_pipeline is None:
+        model = ('fit', nb_classes, use_scaler, 99)
+    else:
+        model = model_pipeline if isinstance(model_pipeline, DeviceClassModel) else model_pipeline.predict_proba
     classes = getattr(model_pipeline, 'classes_', None)
 
     def launch(eng, image):
@@ -452,7 +481,8 @@ def pipe_gray3d_slic_features_model_graphcut(image, nb_classes, dict_features, s
 def segment_resident(d_image, model, dict_features, sp_size=30, sp_regul=0.2, gc_regul=1., gc_edge_type='model'):
     """ the same hot path with the image ALREADY on the device (a cuda tensor [H, W, 3]) and the results left
     there: returns (segm int32 [H, W], segm_soft float64 [H, W, K]) device tensors.  ``model`` is a callable
-    proba_fn(features) or ('fit', nb_classes, use_scaler, max_iter) for the GPU-fitted default GMM. """
+    proba_fn(features), a :class:`graph_cuts.DeviceClassModel` (evaluated on the GPU) or ('fit', nb_classes, use_scaler, max_iter)
+    for the GPU-fitted default GMM. """
     return _run_resident(get_engine(), d_image, model, dict_features, sp_size, sp_regul, gc_regul, gc_edge_type)[:2]
 
 
@@ -494,9 +524,12 @@ def segment_color2d_slic_features_model_graphcut(image, model_pipeline, dict_fea
                                                  gc_edge_type='model', debug_visual=None):
     """ complete pipeline with a given (already fitted) model (reference pipelines.py:160-241)
 
+    :param model_pipeline: a fitted model with ``predict_proba`` (evaluated on the host, as in the reference), or a
+        :class:`graph_cuts.DeviceClassModel` wrapping one (evaluated on the GPU: the path never leaves the device)
     :return tuple(ndarray,ndarray): segmentation [H, W], soft segmentation [H, W, K]
     """
     logging.info('PIPELINE Superpixels-Features-Model-GraphCut')
     classes = getattr(model_pipeline, 'classes_', None)
-    return _segment(image, model_pipeline.predict_proba, dict_features, sp_size, sp_regul, gc_regul, gc_edge_type, debug_visual,
+    model = model_pipeline if isinstance(model_pipeline, DeviceClassModel) else model_pipeline.predict_proba
+    return _segment(image, model, dict_features, sp_size, sp_regul, gc_regul, gc_edge_type, debug_visual,
                     classes=classes)

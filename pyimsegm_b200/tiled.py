@@ -330,9 +330,36 @@ def pipe_color2d_slic_features_model_graphcut_tiled(image, nb_classes, dict_feat
     :return tuple: (segm [rows, W] int32, segm_soft [rows, W, K] float64 or None, (row_lo, row_hi)); with ``gather_segm``
         ``segm`` is the whole [H, W] map on every rank (``segm_soft`` stays banded: it is 8*K bytes per pixel)
     """
+    return _banded_pipeline(image, ('fit', nb_classes, use_scaler, max_iter), dict_features, sp_size, sp_regul, gc_regul,
+                            gc_edge_type, comm, bands_per_rank, want_soft, gather_segm)
+
+
+def segment_color2d_slic_features_model_graphcut_tiled(image, model, dict_features=None, sp_size=30, sp_regul=0.2, gc_regul=1.,
+                                                       gc_edge_type='model', comm=None, bands_per_rank=1, want_soft=True,
+                                                       gather_segm=False):
+    """ ``segment_color2d_slic_features_model_graphcut`` (reference pipelines.py:160-241) -- a model fitted beforehand, e.g. by
+    ``estim_model_classes_group`` on other images -- for one image banded over the GPUs of ``comm``, as
+    :func:`pipe_color2d_slic_features_model_graphcut_tiled`.  The class probabilities are evaluated on the device.
+
+    :param model: a :class:`graph_cuts.DeviceClassModel`, or a fitted mixture model it can wrap (wrapped on entry)
+    :return tuple: (segm [rows, W], segm_soft [rows, W, K] float64 or None, (row_lo, row_hi)); ``segm`` maps through the
+        model's ``classes_`` when it has them
+    """
+    from .graph_cuts import DeviceClassModel
+    model = model if isinstance(model, DeviceClassModel) else DeviceClassModel(model)
+    segm, soft, rows = _banded_pipeline(image, model, dict_features, sp_size, sp_regul, gc_regul, gc_edge_type, comm, bands_per_rank,
+                                        want_soft, gather_segm)
+    classes = getattr(model, 'classes_', None)
+    return (segm if classes is None else np.asarray(classes)[segm]), soft, rows
+
+
+def _banded_pipeline(image, model, dict_features, sp_size, sp_regul, gc_regul, gc_edge_type, comm, bands_per_rank, want_soft,
+                     gather_segm):
+    """the banded pipeline; ``model`` is ('fit', nb_classes, use_scaler, max_iter) -- the default GMM fitted on the device -- or a
+    DeviceClassModel evaluated on the device"""
     from . import graph_cuts
     from .descriptors import flags_are_native, native_feature_layout
-    from .pipelines import _device_graphcut, _soft_on_side_stream
+    from .pipelines import _check_model_width, _device_graphcut, _soft_on_side_stream
     from .superpixels import _as_rgb_like, _supported_dtype, slic_params
     if sp_regul <= 0.:
         raise ValueError('slic. regularisation must be positive')
@@ -349,8 +376,19 @@ def pipe_color2d_slic_features_model_graphcut_tiled(image, nb_classes, dict_feat
     n_seg, compact = slic_params((H, W), sp_size, sp_regul)
     if n_seg < 1:
         raise ValueError('superpixel size %r is larger than the image %r' % (sp_size, tuple(image.shape)))
-    K = int(nb_classes)
-    n_init = max(1, int(np.sqrt(max_iter)))
+    if isinstance(model, graph_cuts.DeviceClassModel):
+        _check_model_width(model, dict_features)
+        d_model = model.device_params(eng)
+
+        def class_proba(res):
+            return eng.gmm_predict(res.d_feat, d_model, model.n_classes, d_n=res.d_n_labels)
+    else:
+        _, K, use_scaler, max_iter = model
+        K = int(K)
+        n_init = max(1, int(np.sqrt(max_iter)))
+
+        def class_proba(res):
+            return eng.gmm_fit_predict(res.d_feat, K, n_init, max_iter, use_scaler, graph_cuts.RANDOM_SEED, d_n=res.d_n_labels)[0]
     force_whole, redo_front, cap = False, True, None
     while True:
         if redo_front:
@@ -358,7 +396,7 @@ def pipe_color2d_slic_features_model_graphcut_tiled(image, nb_classes, dict_feat
                              force_whole=force_whole, raw_margin=margin)
             features_tiled(res, image.dtype, int(image.shape[2]), layout, ncol, comm=comm, eng=eng)
             nb = int(res.nb_bound)
-            d_proba, _ = eng.gmm_fit_predict(res.d_feat, K, n_init, max_iter, use_scaler, graph_cuts.RANDOM_SEED, d_n=res.d_n_labels)
+            d_proba = class_proba(res)          # the model fitted on this image, or the given one evaluated
             redo_front = False
         lo, hi = res.bands[res.local[0]].own_lo, res.bands[res.local[-1]].own_hi
         h_soft = soft_done = None
